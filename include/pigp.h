@@ -255,8 +255,11 @@ int pigp_set_side_stream(int on);
 /* Panel schedule of the factorisation: tiles = 0 is the plain recursion; tiles = W > 0 factors coarse panels of W tile
  * columns on the chain stream and applies each panel to the rest of the matrix on a bulk stream, one panel ahead (the big
  * trailing updates leave the N/128-step dependency chain); tiles < 0 = automatic, which is the default when PIGP_LOOKAHEAD
- * is unset: panels (W = 2 / 4 / 16 by size) for single-GPU NLL-only evaluations of 12 tiles or more -- they have no L^-T
- * work to fill the chain's bubbles -- and the plain recursion otherwise.  Process-global. */
+ * is unset.  The automatic width depends on the tile count T = N/128 and applies to single-GPU evaluations only (sharded
+ * ones keep the plain recursion): NLL-only evaluations (and pigp_predict) have no L^-T work to fill the chain's bubbles
+ * and take W = 2 for 12 <= T < 64, 4 for T < 128 and 16 above; NLL + gradient evaluations take W = 2 for 16 <= T < 32 and
+ * W = 4 for 32 <= T < 96, where the L^-T products leave bubbles that panels still fill.  Otherwise the plain recursion.
+ * Process-global. */
 int pigp_set_lookahead(int tiles);
 int pigp_profile_start(void);
 int pigp_profile_stop(double* ms_out, int64_t* launches_out, double* flops_out);

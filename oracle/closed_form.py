@@ -16,11 +16,39 @@ d/dr_d = d/ds and d/dr'_d = -d/ds.  An operator is a polynomial in
 
 ``oracle.autodiff_ops`` (the literal restatement) is the check for this file:
 tests/test_oracle.py compares every operator, both forms, 1-/2-/3-D.
-This is test infrastructure (see oracle/__init__.py).
+This is test infrastructure (see oracle/__init__.py).  eval_operator also takes torch tensors for the points (same
+formulas, float64 on their device), so that large float64 references can be evaluated on a GPU.
 """
 import itertools
 
 import numpy as np
+
+
+def _is_torch(x):
+    return type(x).__module__.startswith("torch")
+
+
+def _exp_for(x):
+    if _is_torch(x):
+        import torch
+
+        return torch.exp
+    return np.exp
+
+
+def _prod(factors):
+    out = factors[0]
+    for f in factors[1:]:
+        out = out * f
+    return out
+
+
+def _stack(arrs):
+    if _is_torch(arrs[0]):
+        import torch
+
+        return torch.stack(arrs)
+    return np.stack(arrs)
 
 
 def _e(i, dim):
@@ -60,7 +88,7 @@ def operator_polynomial(name, dim):
 def _g(n, s, a):
     t = a * s * s
     if n == 0:
-        return np.ones_like(s)
+        return s * 0.0 + 1.0
     if n == 1:
         return -a * s
     if n == 2:
@@ -76,7 +104,7 @@ def _dg_da(n, s, a):
     """d g_n / d a."""
     s2 = s * s
     if n == 0:
-        return np.zeros_like(s)
+        return s * 0.0
     if n == 1:
         return -s
     if n == 2:
@@ -89,8 +117,9 @@ def _dg_da(n, s, a):
 
 
 def _prep(r, rp, dim, dtype=np.float64):
-    r = np.asarray(r, dtype=dtype)
-    rp = np.asarray(rp, dtype=dtype)
+    if not _is_torch(r):
+        r = np.asarray(r, dtype=dtype)
+        rp = np.asarray(rp, dtype=dtype)
     if dim == 1:
         r = r.reshape(-1, 1)
         rp = rp.reshape(-1, 1)
@@ -107,8 +136,11 @@ def eval_operator(name, r, rp, theta, form, dim, with_grad=False, dtype=np.float
     theta = np.asarray(theta, dtype=dtype)
     gamma = np.exp(theta[0])
     a = np.exp(-2.0 * theta[1:1 + dim])
+    if _is_torch(r):  # plain floats: a numpy scalar on the left of a tensor product would convert the tensor
+        gamma, a = float(gamma), [float(x) for x in a]
     s = _prep(r, rp, dim, dtype)
-    E = [np.exp(-0.5 * a[d] * s[d] * s[d]) for d in range(dim)]
+    exp = _exp_for(s[0])
+    E = [exp(-0.5 * a[d] * s[d] * s[d]) for d in range(dim)]
 
     def G(n, d):
         return _g(n, s[d], a[d]) * E[d]
@@ -117,20 +149,20 @@ def eval_operator(name, r, rp, theta, form, dim, with_grad=False, dtype=np.float
         # d/dlogl = -2a d/da ; d(g E)/da = (dg/da - s^2/2 g) E
         return -2.0 * a[d] * (_dg_da(n, s[d], a[d]) - 0.5 * s[d] * s[d] * _g(n, s[d], a[d])) * E[d]
 
-    val = np.zeros_like(s[0])
-    grad = np.zeros((1 + dim,) + s[0].shape, dtype=dtype) if with_grad else None
+    val = s[0] * 0.0
+    grad = [s[0] * 0.0 for _ in range(1 + dim)] if with_grad else None
     for coef, alpha, beta in operator_polynomial(name, dim):
         sign = coef * (-1.0) ** sum(beta)
         order = _add(alpha, beta)
         if form == "product":
             factors = [G(order[d], d) for d in range(dim)]
-            term = sign * gamma * np.prod(factors, axis=0)
+            term = sign * gamma * _prod(factors)
             val += term
             if with_grad:
                 grad[0] += term
                 for e in range(dim):
                     others = [factors[d] for d in range(dim) if d != e]
-                    rest = np.prod(others, axis=0) if others else 1.0
+                    rest = _prod(others) if others else 1.0
                     grad[1 + e] += sign * gamma * dG_dlogl(order[e], e) * rest
         elif form == "additive":
             active = [d for d in range(dim) if order[d] > 0]
@@ -150,4 +182,6 @@ def eval_operator(name, r, rp, theta, form, dim, with_grad=False, dtype=np.float
                     grad[1 + e] += sign * gamma * dG_dlogl(order[e], e)
         else:
             raise ValueError(form)
+    if with_grad:
+        grad = _stack(grad)
     return (val, grad) if with_grad else val

@@ -666,6 +666,11 @@ int launch_gemm(const GemmDesc& g_in, cudaStream_t st) {
         set_error("pigp gemm: M, N and K must be multiples of 128");
         return PIGP_EINVAL;
     }
+    // the operand loads are 16-byte cp.async copies of element pairs: every row must start 16-byte aligned
+    if (g.lda % 2 || g.ldb % 2 || g.ldc % 2 || (g.Lkk && g.ldl % 2)) {
+        set_error("pigp gemm: lda, ldb and ldc must be even");
+        return PIGP_EINVAL;
+    }
     if (g.m_ts == 0) g.m_ts = 1;
     if (g.Lkk) {
         if (g.N != BM || g.K != BM || !g.a_kcontig || !g.b_kcontig || g.C != g.A || g.alpha != 1.0 || g.beta != 0.0) {
