@@ -13,7 +13,9 @@
  * their inputs to the device and their results back, and synchronise the
  * stream before returning; the others never synchronise.
  *
- * Threads: the device-pointer entry points (pigp_assemble, pigp_assemble_diag) only read a plan, so one plan may serve
+ * Threads: the device-pointer entry points (pigp_assemble, pigp_assemble_diag, and the test building blocks
+ * pigp_assemble_owned and pigp_trace_grad, whose tile lists and partial sums are stream-ordered allocations on the
+ * caller's stream) only read a plan, so one plan may serve
  * several threads / streams at once.  pigp_plan_set_points_host and every _host entry point use staging buffers owned by
  * the plan or the solver and are NOT thread-safe per handle.  A solver (pigp_solver / pigp_dsolver) owns its workspace and
  * must be used by one thread at a time -- use one solver per thread / stream.  Every entry point switches the calling
@@ -207,6 +209,16 @@ int pigp_potri_lower(const double* L_dev, int64_t ld, int64_t n, const double* i
 int pigp_dgemm(int M, int N, int K, double alpha, const double* A_dev, int64_t lda, int a_kcontig,
                const double* B_dev, int64_t ldb, int b_kcontig, double beta, double* C_dev, int64_t ldc,
                int lower_only, void* stream);
+/* The lower-triangle entries of the 128-row tiles of a symmetric plan's matrix that `rank` owns (tile t belongs to rank
+ * t mod world), over exactly the tile list the block-cyclic solver assembles into (64-row tiles, or 16-row tiles when
+ * that leaves fewer than two per SM).  Nothing else of K_dev (ld >= cols) is written. */
+int pigp_assemble_owned(const pigp_plan* plan, int rank, int world, const double* theta_dev, double eps, int add_diag,
+                        double* K_dev, int64_t ld, void* stream);
+/* The solver's fused trace gradient over the same owned tiles:  grad[p] = 1/2 sum_jk w_jk (X_jk - alpha_j alpha_k)
+ * dK_jk/dtheta_p  over the owned lower entries, w = 1 on the diagonal and 2 below it (X is read below the diagonal only;
+ * any 8-byte-aligned X_dev).  Summing grad over the ranks of a world gives the world = 1 result. */
+int pigp_trace_grad(const pigp_plan* plan, int rank, int world, const double* theta_dev, const double* X_dev, int64_t ld,
+                    const double* alpha_dev, double* grad_dev, void* stream);
 
 /* --- multi-GPU evaluation (new; the reference is single device).  One pigp_dsolver per rank; 128-row tile t of K
  * belongs to rank t mod world.  Ranks exchange data by stores into each other's slab over NVLink (P2P) and epoch flags;

@@ -77,6 +77,10 @@ _SIGNATURES = {
     "pigp_potri_lower": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "pigp_dgemm": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_double, C.c_void_p, C.c_int64, C.c_int, C.c_void_p, C.c_int64,
                              C.c_int, C.c_double, C.c_void_p, C.c_int64, C.c_int, C.c_void_p]),
+    "pigp_assemble_owned": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_double, C.c_int, C.c_void_p, C.c_int64,
+                                      C.c_void_p]),
+    "pigp_trace_grad": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p,
+                                  C.c_void_p]),
     "pigp_dsolver_create": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.POINTER(C.c_void_p)]),
     "pigp_dsolver_destroy": (None, [C.c_void_p]),
     "pigp_dsolver_slab": (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_int64)]),

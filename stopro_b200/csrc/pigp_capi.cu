@@ -759,4 +759,63 @@ int pigp_dgemm(int M, int N, int K, double alpha, const double* A_dev, int64_t l
     return launch_gemm(g, as_stream(stream));
 }
 
+// The owned lower tiles of build_lower_tiles_owned in a stream-ordered device buffer (freed by the caller with
+// cudaFreeAsync on the same stream), so that neither entry point below synchronises.
+static int owned_tiles(const pigp_plan* p, int rank, int world, cudaStream_t st, AsmTile** dev, int64_t* n) {
+    std::vector<AsmTile> v;
+    build_lower_tiles_owned(p, rank, world, v);
+    *n = (int64_t)v.size();
+    *dev = nullptr;
+    if (v.empty()) return PIGP_OK;
+    PIGP_CUDA(cudaMallocAsync(reinterpret_cast<void**>(dev), v.size() * sizeof(AsmTile), st));
+    const cudaError_t e = cudaMemcpyAsync(*dev, v.data(), v.size() * sizeof(AsmTile), cudaMemcpyHostToDevice, st);
+    if (e != cudaSuccess) {
+        cudaFreeAsync(*dev, st);
+        *dev = nullptr;
+        PIGP_CUDA(e);
+    }
+    return PIGP_OK;
+}
+
+int pigp_assemble_owned(const pigp_plan* p, int rank, int world, const double* theta_dev, double eps, int add_diag,
+                        double* K_dev, int64_t ld, void* stream) {
+    if (!p || !p->symmetric || !theta_dev || !K_dev || world < 1 || rank < 0 || rank >= world || ld < p->cols) {
+        set_error("pigp_assemble_owned: needs a symmetric plan, 0 <= rank < world, ld >= cols and device buffers");
+        return PIGP_EINVAL;
+    }
+    PIGP_TRY(use_device(p));
+    const cudaStream_t st = as_stream(stream);
+    AsmTile* tiles = nullptr;
+    int64_t n = 0;
+    PIGP_TRY(owned_tiles(p, rank, world, st, &tiles, &n));
+    const int rc = launch_assemble(p, tiles, n, theta_dev, eps, add_diag, K_dev, ld, st);
+    if (tiles) PIGP_CUDA(cudaFreeAsync(tiles, st));
+    return rc;
+}
+
+int pigp_trace_grad(const pigp_plan* p, int rank, int world, const double* theta_dev, const double* X_dev, int64_t ld,
+                    const double* alpha_dev, double* grad_dev, void* stream) {
+    if (!p || !p->symmetric || !theta_dev || !X_dev || !alpha_dev || !grad_dev || world < 1 || rank < 0 || rank >= world ||
+        ld < p->cols) {
+        set_error("pigp_trace_grad: needs a symmetric plan, 0 <= rank < world, ld >= cols and device buffers");
+        return PIGP_EINVAL;
+    }
+    PIGP_TRY(use_device(p));
+    const cudaStream_t st = as_stream(stream);
+    AsmTile* tiles = nullptr;
+    int64_t n = 0;
+    PIGP_TRY(owned_tiles(p, rank, world, st, &tiles, &n));
+    double* partials = nullptr;
+    int rc = PIGP_OK;
+    const cudaError_t e = cudaMallocAsync(reinterpret_cast<void**>(&partials), sizeof(double) * MAX_THETA * std::max<int64_t>(n, 1), st);
+    if (e != cudaSuccess) {
+        set_error(std::string("pigp_trace_grad: cudaMallocAsync: ") + cudaGetErrorString(e));
+        rc = PIGP_ECUDA;
+    }
+    if (rc == PIGP_OK) rc = launch_grad(p, tiles, n, theta_dev, X_dev, ld, alpha_dev, partials, grad_dev, st);
+    if (partials) cudaFreeAsync(partials, st);
+    if (tiles) cudaFreeAsync(tiles, st);
+    return rc;
+}
+
 }  // extern "C"

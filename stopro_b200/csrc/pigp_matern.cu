@@ -21,18 +21,20 @@ __constant__ double c_mat[3][5][2][6];
 __constant__ double c_kappa[3];
 
 static void poly_tables(double out[3][5][2][6], double kappa[3]) {
-    const double base[3][5] = {{1.0, 1.0, 1.0 / 3.0, 0.0, 0.0},
-                               {1.0, 1.0, 2.0 / 5.0, 1.0 / 15.0, 0.0},
-                               {1.0, 1.0, 3.0 / 7.0, 2.0 / 21.0, 1.0 / 105.0}};
+    // q scaled by a common denominator, so that the recurrences run on exact integers: a coefficient that is 0 (the
+    // constant term of q_3 for mt52 and mt72, which makes the third derivative vanish at s = 0) stays exactly 0, and every
+    // other one is rounded once, by the final division
+    const double base[3][5] = {{3, 3, 1, 0, 0}, {15, 15, 6, 1, 0}, {105, 105, 45, 10, 1}};
+    const double denom[3] = {3, 15, 105};
     kappa[0] = sqrt(5.0); kappa[1] = sqrt(7.0); kappa[2] = 3.0;
     for (int k = 0; k < 3; ++k) {
         double q[6] = {base[k][0], base[k][1], base[k][2], base[k][3], base[k][4], 0.0};
         for (int n = 0; n < 5; ++n) {
             double dq[6] = {0, 0, 0, 0, 0, 0};
             for (int i = 0; i < 5; ++i) dq[i] = (i + 1) * q[i + 1];
-            for (int i = 0; i < 6; ++i) out[k][n][0][i] = q[i];
+            for (int i = 0; i < 6; ++i) out[k][n][0][i] = q[i] / denom[k];
             // u = -n q + rho (q - q')
-            for (int i = 0; i < 6; ++i) out[k][n][1][i] = -n * q[i] + (i > 0 ? q[i - 1] - dq[i - 1] : 0.0);
+            for (int i = 0; i < 6; ++i) out[k][n][1][i] = (-n * q[i] + (i > 0 ? q[i - 1] - dq[i - 1] : 0.0)) / denom[k];
             for (int i = 0; i < 6; ++i) q[i] = dq[i] - q[i];  // q_{n+1}
         }
     }

@@ -11,39 +11,10 @@ import numpy as np
 import pytest
 
 from oracle import blocks_ref, closed_form
+from oracle.desc_ref import eval_desc
 from stopro_b200 import _lib, operators
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-
-
-
-def eval_desc_numpy(desc, dim, r, rp, theta, lbox=None):
-    """Host (numpy) evaluation of one pigp_block_desc: test helper to check the descriptor compiler against the
-    oracle's hand-written block tables without a GPU."""
-    r = np.asarray(r, dtype=np.float64).reshape(len(r), dim)
-    rp = np.asarray(rp, dtype=np.float64).reshape(len(rp), dim)
-    theta = np.asarray(theta, dtype=np.float64)
-    lb = np.zeros(dim) if lbox is None else np.asarray(lbox, dtype=np.float64)[:dim]
-
-    def G(n, s, a):
-        t = a * s * s
-        g = [1.0, -a * s, a * (t - 1.0), a * a * s * (3.0 - t), a * a * (t * t - 6.0 * t + 3.0)][n]
-        return g * np.exp(-0.5 * t)
-
-    out = np.zeros((len(r), len(rp)))
-    for sf in range(desc.shift_first + 1):
-        for ss in range(desc.shift_second + 1):
-            sign = -1.0 if (desc.shift_first - sf + desc.shift_second - ss) % 2 else 1.0
-            s = [(r[:, None, d] + sf * lb[d]) - (rp[None, :, d] + ss * lb[d]) for d in range(dim)]
-            for k in range(desc.n_terms):
-                t = desc.terms[k]
-                th = theta[t.group * (1 + dim):(t.group + 1) * (1 + dim)]
-                val = t.coef * np.exp(th[0]) * np.ones_like(out)
-                for d in range(dim):
-                    if t.order[d] >= 0:
-                        val = val * G(t.order[d], s[d], np.exp(-2.0 * th[1 + d]))
-                out += sign * val
-    return out
 
 
 @pytest.fixture(scope="session")
@@ -109,7 +80,7 @@ def test_descriptor_compiler_reproduces_the_block_library(dim, form):
         if name in ("Kuydifux",):  # reference quirk: built from Kuxuy == 0 (gp_2D_stokes_independent.py:164-165)
             assert not want.any()
         desc = operators.make_desc(oa, ob, fields, dim, form == "product")
-        got = eval_desc_numpy(desc, dim, r, rp, theta, lbox)
+        got = eval_desc(desc, dim, r, rp, theta, lbox, product=form == "product")
         scale = max(np.max(np.abs(want)), 1.0)
         assert np.max(np.abs(got - want)) <= 1e-12 * scale, name
         checked += 1
@@ -122,7 +93,7 @@ def test_scalar_models_descriptors():
     r, rp, theta = rng.random(6), rng.random(5), np.array([0.2, -0.3])
     for a, b, op in [("y", "y", "K"), ("y", "ly", "L1K"), ("ly", "ly", "LLK")]:
         desc = operators.make_desc(obs[a], obs[b], fields, 1, True)
-        got = eval_desc_numpy(desc, 1, r, rp, theta)
+        got = eval_desc(desc, 1, r, rp, theta)
         want = closed_form.eval_operator(op, r, rp, theta, "product", 1)
         assert np.max(np.abs(got - want)) <= 1e-13 * np.max(np.abs(want))
 

@@ -5,8 +5,8 @@ import numpy as np
 import pytest
 
 from oracle import blocks_ref, closed_form
+from oracle.desc_ref import eval_desc
 from stopro_b200 import synthetic
-from test_host import eval_desc_numpy
 from stopro_b200 import operators
 
 MODELS = {
@@ -49,7 +49,7 @@ def test_class_tables_match_the_reference_tables(name):
     def check(obs_a, obs_b, block_name, zero=False):
         want = blocks_ref.eval_block(block_name, table, op_eval, r, rp, theta, lbox, lambda n, m: np.zeros((n, m)))
         desc = operators.make_desc(obs_a, obs_b, gp._fields, dim, gp.product_form)
-        got = np.zeros_like(want) if zero else eval_desc_numpy(desc, dim, r, rp, theta, lbox)
+        got = np.zeros_like(want) if zero else eval_desc(desc, dim, r, rp, theta, lbox, product=gp.product_form)
         assert np.max(np.abs(got - want)) <= 1e-12 * max(np.max(np.abs(want)), 1.0), (name, block_name)
 
     tr = gp._observables(gp.train_observables)
