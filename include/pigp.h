@@ -164,7 +164,10 @@ int pigp_nll_grad_host(pigp_solver* s, const double* theta_host, const double* p
 
 /* predictingFunction_all (GP/gp.py:226-256, postGP :91-120).  mixed: rows = test points, cols = training points;
  * test: symmetric plan over the test points.  mu_dev[M] = K_ab K_bb^-1 y (mu_test is added by the caller);
- * cov_dev: full M x M posterior covariance K_aa - V^T V (ld = M) when want_full_cov, else its diagonal (M). */
+ * cov_dev: full M x M posterior covariance K_aa - V^T V (ld = M) when want_full_cov, else its diagonal (M).
+ * PIGP_EINVAL before any launch when mixed is not (M x N training points), test is not symmetric over the M test points,
+ * or either plan's dim, kernel_type, product_form or n_groups differs from the training plan's (both read theta as the
+ * training plan lays it out, noise entry excepted). */
 int pigp_predict(pigp_solver* s, const pigp_plan* mixed, const pigp_plan* test, const double* theta_dev,
                  const double* y_dev, double eps, double* mu_dev, double* cov_dev, int want_full_cov,
                  int32_t* info_dev, void* stream);

@@ -597,6 +597,12 @@ int pigp_predict(pigp_solver* s, const pigp_plan* mixed, const pigp_plan* test, 
         set_error("pigp_predict: mixed must be (test x train) and test symmetric over the same test points");
         return PIGP_EINVAL;
     }
+    for (const pigp_plan* p : {mixed, test})
+        if (p->dim != s->plan->dim || p->kernel_type != s->plan->kernel_type || p->product_form != s->plan->product_form ||
+            p->n_groups != s->plan->n_groups) {
+            set_error("pigp_predict: mixed and test plans must have the training plan's dim, kernel_type, product_form and n_groups");
+            return PIGP_EINVAL;
+        }
     PIGP_TRY(use_device(s->plan));
     cudaStream_t st = as_stream(stream);
     int32_t* info = info_dev ? info_dev : s->info;
