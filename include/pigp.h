@@ -200,7 +200,9 @@ int pigp_adam_host(pigp_solver* s, const double* theta0_host, const double* y_ho
 /* In-place lower Cholesky of the leading n x n of A (row-major, ld), applying L^-T to the m_extra rows below it
  * (jnp.linalg.cholesky + jnp.linalg.solve of GP/gp.py:83-84, :106-118).  invd_dev: n/128 inverse diagonal tiles
  * (128*128 doubles each), workspace output.  Only the lower triangle of A is defined on output (the part above the
- * diagonal is not referenced by any consumer and is left partly overwritten). */
+ * diagonal is not referenced by any consumer and is left partly overwritten).  Runs the solver's factorisation with the
+ * panel width of an NLL-only evaluation (pigp_set_lookahead); the panel schedule's bulk stream is one per device,
+ * shared by the calling threads. */
 int pigp_potrf_lower(double* A_dev, int64_t ld, int64_t n, int64_t m_extra, double* invd_dev,
                      int32_t* info_dev, void* stream);
 /* K^-1 (lower triangle, into X_dev) from the factor L (lower of L_dev) -- replaces solve(L.T, solve(L, I)),
@@ -267,14 +269,14 @@ int64_t pigp_launch_count(void);
 /* on = 1 (default): the Y = L^-T products run on a side stream concurrently with the Cholesky chain.  on = 0 puts every
  * kernel on one stream, so that per-launch event times do not overlap (used by the per-class timing pass of bench.py). */
 int pigp_set_side_stream(int on);
-/* Panel schedule of the factorisation: tiles = 0 is the plain recursion; tiles = W > 0 factors coarse panels of W tile
- * columns on the chain stream and applies each panel to the rest of the matrix on a bulk stream, one panel ahead (the big
- * trailing updates leave the N/128-step dependency chain); tiles < 0 = automatic, which is the default when PIGP_LOOKAHEAD
- * is unset.  The automatic width depends on the tile count T = N/128 and applies to single-GPU evaluations only (sharded
- * ones keep the plain recursion): NLL-only evaluations (and pigp_predict) have no L^-T work to fill the chain's bubbles
- * and take W = 2 for 12 <= T < 64, 4 for T < 128 and 16 above; NLL + gradient evaluations take W = 2 for 16 <= T < 32 and
- * W = 4 for 32 <= T < 96, where the L^-T products leave bubbles that panels still fill.  Otherwise the plain recursion.
- * Process-global. */
+/* Panel schedule of the factorisation (solver evaluations and pigp_potrf_lower): tiles = 0 is the plain recursion;
+ * tiles = W > 0 factors coarse panels of W tile columns on the chain stream and applies each panel to the rest of the
+ * matrix on a bulk stream, one panel ahead (the big trailing updates leave the N/128-step dependency chain); tiles < 0 =
+ * automatic, which is the default when PIGP_LOOKAHEAD is unset.  The automatic width depends on the tile count T = N/128
+ * and applies to single-GPU evaluations only (sharded ones keep the plain recursion): NLL-only evaluations (and
+ * pigp_predict and pigp_potrf_lower) have no L^-T work to fill the chain's bubbles and take W = 2 for 12 <= T < 64, 4 for
+ * T < 128 and 16 above; NLL + gradient evaluations take W = 2 for 16 <= T < 32 and W = 4 for 32 <= T < 96, where the
+ * L^-T products leave bubbles that panels still fill.  Otherwise the plain recursion.  Process-global. */
 int pigp_set_lookahead(int tiles);
 int pigp_profile_start(void);
 int pigp_profile_stop(double* ms_out, int64_t* launches_out, double* flops_out);

@@ -12,11 +12,9 @@
 // * k_potf2: one CTA factors a 128 x 128 diagonal tile in shared memory (32 x 32 blocks: one warp eliminates column pairs,
 //   a second warp inverts the block behind it); k_tile_inv completes inverse tiles off the critical path.
 // * k_trsm_blk: the panel solve X = A inv(L_kk)^T by block forward substitution with refined 32 x 32 diagonal solves.
-// * Host drivers: recursive right-looking Cholesky (all flops in k_gemm), TRTRI + LAUUM for K^-1.
+// * Host drivers: TRTRI + LAUUM for K^-1.  The Cholesky that drives k_potf2, k_trsm_blk and k_gemm is in pigp_dist.cu.
 #include <algorithm>
 #include <cstdlib>
-#include <mutex>
-#include <vector>
 
 #include "pigp_internal.cuh"
 
@@ -1151,114 +1149,6 @@ int launch_potf2(double* A, int64_t ld, double* invd, int32_t* info, int base, c
     return PIGP_OK;
 }
 
-// Factor A[0:n,0:n] and apply L^-T from the right to the m_below rows under it (recursive right-looking).
-static int chol_rec(double* A, int64_t ld, int64_t n, int64_t m_below, double* invd, int32_t* info, int base,
-                    cudaStream_t st) {
-    if (n == TILE) {
-        PIGP_TRY(launch_potf2(A, ld, invd, info, base, st));
-        if (m_below > 0) {
-            // B <- B * inv(L)^T, in place: every CTA reads its own 128 rows completely before writing them
-            GemmDesc g{};
-            g.M = (int)m_below; g.N = TILE; g.K = TILE;
-            g.alpha = 1.0; g.beta = 0.0;
-            g.A = A + TILE * ld; g.lda = ld; g.a_kcontig = 1;
-            g.B = invd; g.ldb = TILE; g.b_kcontig = 1;
-            g.C = A + TILE * ld; g.ldc = ld;
-            g.force_bn128 = 1;
-            g.Lkk = A; g.ldl = ld;
-            PIGP_TRY(launch_gemm(g, st));
-        }
-        return PIGP_OK;
-    }
-    const int64_t n1 = (n / TILE / 2) * TILE, n2 = n - n1;
-    PIGP_TRY(chol_rec(A, ld, n1, n2 + m_below, invd, info, base, st));
-    {
-        // A22 (lower) and every row below it:  C -= A21 * A21^T
-        GemmDesc g{};
-        g.M = (int)(n2 + m_below); g.N = (int)n2; g.K = (int)n1;
-        g.alpha = -1.0; g.beta = 1.0;
-        g.A = A + n1 * ld; g.lda = ld; g.a_kcontig = 1;
-        g.B = A + n1 * ld; g.ldb = ld; g.b_kcontig = 1;
-        g.C = A + n1 * ld + n1; g.ldc = ld;
-        g.lower_only = 1;
-        g.gen = 1; g.m_ts = 1;  // tile-indexed form (row tile 0 = column tile 0): eligible for the small-tile kernels
-        PIGP_TRY(launch_gemm(g, st));
-    }
-    return chol_rec(A + n1 * ld + n1, ld, n2, m_below, invd + (n1 / TILE) * TILE * TILE, info, base + (int)n1, st);
-}
-
-// Panel schedule with look-ahead for the stand-alone factorisation (the solver has its own, pigp_dist.cu): coarse panels
-// of W tile columns, the recursion inside a panel (and its TRSM of all rows below) on the caller's stream, the panel's
-// update of the columns to its right on a bulk stream -- the next panel's columns first, the chain waits only for those.
-struct PanelStreams { cudaStream_t bulk = nullptr; std::vector<cudaEvent_t> pan, next; cudaEvent_t done = nullptr; };
-static PanelStreams g_panel_streams[64];  // per device; the enqueue below holds g_panel_mutex (host threads share them)
-static std::mutex g_panel_mutex;
-
-static int panel_update_dense(double* A, int64_t ld, int64_t rows, int64_t j0, int64_t j1, int64_t c0, int64_t c1, cudaStream_t st) {
-    // C[c0.., [c0, c1)] -= L[c0.., [j0, j1)] L[[c0, c1), [j0, j1)]^T for all `rows` rows from c0 down (lower part)
-    if (c1 <= c0) return PIGP_OK;
-    GemmDesc g{};
-    g.M = (int)(rows - c0); g.N = (int)(c1 - c0); g.K = (int)(j1 - j0);
-    g.alpha = -1.0; g.beta = 1.0;
-    g.A = A + c0 * ld + j0; g.lda = ld; g.a_kcontig = 1;
-    g.B = A + c0 * ld + j0; g.ldb = ld; g.b_kcontig = 1;
-    g.C = A + c0 * ld + c0; g.ldc = ld;
-    g.lower_only = 1;
-    g.gen = 1; g.m_ts = 1;
-    return launch_gemm(g, st);
-}
-
-static int chol_panels(double* A, int64_t ld, int64_t n, int64_t m_extra, double* invd, int32_t* info, int W, cudaStream_t st) {
-    int dev = 0;
-    PIGP_CUDA(cudaGetDevice(&dev));
-    std::lock_guard<std::mutex> lock(g_panel_mutex);
-    PanelStreams& ps = g_panel_streams[dev & 63];
-    const int T = (int)(n / TILE), n_pan = (T + W - 1) / W;
-    if (!ps.bulk) {
-        PIGP_CUDA(cudaStreamCreateWithFlags(&ps.bulk, cudaStreamNonBlocking));
-        PIGP_CUDA(cudaEventCreateWithFlags(&ps.done, cudaEventDisableTiming));
-    }
-    while ((int)ps.pan.size() < n_pan) {
-        cudaEvent_t a = nullptr, b = nullptr;
-        PIGP_CUDA(cudaEventCreateWithFlags(&a, cudaEventDisableTiming));
-        PIGP_CUDA(cudaEventCreateWithFlags(&b, cudaEventDisableTiming));
-        ps.pan.push_back(a);
-        ps.next.push_back(b);
-    }
-    const int64_t rows = n + m_extra, w = (int64_t)W * TILE;
-    // the bulk stream starts behind everything already queued on the caller's stream
-    PIGP_CUDA(cudaEventRecord(ps.done, st));
-    PIGP_CUDA(cudaStreamWaitEvent(ps.bulk, ps.done, 0));
-    for (int64_t j0 = 0, p = 0; j0 < n; j0 += w, ++p) {
-        const int64_t j1 = std::min(j0 + w, n);
-        PIGP_TRY(chol_rec(A + j0 * ld + j0, ld, j1 - j0, rows - j1, invd + (j0 / TILE) * TILE * TILE, info, (int)j0, st));
-        if (j1 >= rows) break;
-        PIGP_CUDA(cudaEventRecord(ps.pan[p], st));
-        PIGP_CUDA(cudaStreamWaitEvent(ps.bulk, ps.pan[p], 0));
-        const int64_t jn = std::min(j1 + w, n);
-        if (j1 < n) PIGP_TRY(panel_update_dense(A, ld, rows, j0, j1, j1, jn, ps.bulk));
-        PIGP_CUDA(cudaEventRecord(ps.next[p], ps.bulk));
-        if (jn < n) PIGP_TRY(panel_update_dense(A, ld, rows, j0, j1, jn, n, ps.bulk));
-        PIGP_CUDA(cudaStreamWaitEvent(st, ps.next[p], 0));
-    }
-    PIGP_CUDA(cudaEventRecord(ps.done, ps.bulk));
-    PIGP_CUDA(cudaStreamWaitEvent(st, ps.done, 0));
-    return PIGP_OK;
-}
-
-int potrf_lower(double* A, int64_t ld, int64_t n, int64_t m_extra, double* invd, int32_t* info, cudaStream_t st) {
-    if (n <= 0 || n % TILE || m_extra % TILE || m_extra < 0 || ld % 2) {
-        set_error("pigp potrf: n and m_extra must be multiples of 128 and ld even");
-        return PIGP_EINVAL;
-    }
-    const int T = (int)(n / TILE);
-    const int W = T < 12 ? 0 : T < 64 ? 2 : T < 128 ? 4 : 16;  // same rule as the solver's NLL-only evaluation
-    if (W > 0) PIGP_TRY(chol_panels(A, ld, n, m_extra, invd, info, W, st));
-    else PIGP_TRY(chol_rec(A, ld, n, m_extra, invd, info, 0, st));
-    // the factorisation leaves the diagonal 32-blocks of the inverse tiles; callers of this entry point get complete tiles
-    return launch_tile_inv(A, ld, invd, 0, 1, (int)(n / TILE), nullptr, 0, st, 1);
-}
-
 // ----------------------------------------------------------------------------------------------- TRTRI + LAUUM
 __global__ void k_place_diag(double* W, int64_t ld, const double* invd) {
     // diagonal tile b of W <- invd[b] (full tile, zeros above the diagonal)
@@ -1359,50 +1249,6 @@ int launch_logdet_quad(const double* A, int64_t ld, int64_t n, const double* v, 
     return PIGP_OK;
 }
 
-// y[j] = sum_{i >= j} W[i][j] x[i].  Pass 1: CTA (column block, row chunk) sums its rows into part[chunk][j]
-// (coalesced 1 KB row segments, 4 rows in flight per thread); pass 2 adds the chunks in order (deterministic).
-constexpr int TRMV_CHUNK = 1024;
-__global__ void __launch_bounds__(256) k_trmv_lower_t(const double* W, int64_t ld, int64_t n, const double* x, double* part) {
-    __shared__ double sh[2][128];
-    const int c = threadIdx.x & 127, h = threadIdx.x >> 7;
-    const int64_t j0 = (int64_t)blockIdx.x * 128, j = j0 + c;
-    const int64_t r0 = max((long long)blockIdx.y * TRMV_CHUNK, (long long)j0);
-    const int64_t r1 = min(((long long)blockIdx.y + 1) * TRMV_CHUNK, (long long)n);
-    double s0 = 0.0, s1 = 0.0, s2 = 0.0, s3 = 0.0;
-    if (j < n) {
-        int64_t i = r0 + h;
-        for (; i + 6 < r1; i += 8) {
-            const double w0 = W[i * ld + j], w1 = W[(i + 2) * ld + j], w2 = W[(i + 4) * ld + j], w3 = W[(i + 6) * ld + j];
-            if (i >= j) s0 = fma(w0, x[i], s0);
-            if (i + 2 >= j) s1 = fma(w1, x[i + 2], s1);
-            if (i + 4 >= j) s2 = fma(w2, x[i + 4], s2);
-            if (i + 6 >= j) s3 = fma(w3, x[i + 6], s3);
-        }
-        for (; i < r1; i += 2)
-            if (i >= j) s0 = fma(W[i * ld + j], x[i], s0);
-    }
-    sh[h][c] = (s0 + s1) + (s2 + s3);
-    __syncthreads();
-    if (h == 0 && j < n) part[(int64_t)blockIdx.y * n + j] = sh[0][c] + sh[1][c];
-}
-__global__ void __launch_bounds__(256) k_sum_chunks(const double* part, int64_t n, int n_chunks, double* y) {
-    const int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (j >= n) return;
-    double s = 0.0;
-    for (int c = (int)(j / TRMV_CHUNK); c < n_chunks; ++c) s += part[(int64_t)c * n + j];
-    y[j] = s;
-}
-
-int launch_trmv_lower_t(const double* W, int64_t ld, int64_t n, const double* x, double* y, double* part, cudaStream_t st) {
-    const int n_chunks = (int)((n + TRMV_CHUNK - 1) / TRMV_CHUNK);
-    ProfScope prof(PROF_MISC, st);
-    k_trmv_lower_t<<<dim3((unsigned)((n + 127) / 128), (unsigned)n_chunks), 256, 0, st>>>(W, ld, n, x, part);
-    k_sum_chunks<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(part, n, n_chunks, y);
-    count_launch(2);
-    PIGP_CUDA(cudaGetLastError());
-    return PIGP_OK;
-}
-
 // y[i] = sum_j A[i][j] x[j]: one warp per row
 __global__ void __launch_bounds__(256) k_gemv(const double* A, int64_t ld, int64_t m, int64_t n, const double* x, double* y) {
     const int64_t row = (int64_t)blockIdx.x * 8 + (threadIdx.x >> 5);
@@ -1454,8 +1300,6 @@ int preload_dense() {
     PIGP_PRELOAD(k_tile_inv);
     PIGP_PRELOAD(k_place_diag);
     PIGP_PRELOAD(k_logdet_quad);
-    PIGP_PRELOAD(k_trmv_lower_t);
-    PIGP_PRELOAD(k_sum_chunks);
     PIGP_PRELOAD(k_gemv);
     return PIGP_OK;
 }

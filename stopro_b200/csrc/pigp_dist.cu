@@ -16,9 +16,11 @@
 //     peer stores and summed in rank order (deterministic, identical on every rank);
 //   * log-det, |L^-1 y|^2 and alpha = K^-1 y are computed redundantly from the replicated L / Y; each rank carries its
 //     own y row tile (placed at the first tile index >= npad/128 that it owns) through the TRSMs.
+// The factorisation (leaf, rec, chol_lookahead over a FactorView) is also pigp_potrf_lower's, on one rank.
 #include <algorithm>
 #include <cstdlib>
 #include <cstring>
+#include <mutex>
 
 #include "pigp_internal.cuh"
 
@@ -188,6 +190,38 @@ __global__ void k_copy_v(const double* row, int64_t npad, double* v) {
     if (i < npad) v[i] = row[i];
 }
 
+// Streams and events of the panel schedule (chol_lookahead): the bulk stream of the trailing updates, per coarse panel
+// "chain done" and "next panel's columns updated", and the event that joins the bulk stream back.  Grows on demand.
+struct PanelSched {
+    bool low_priority = false;  // the solver's bulk stream yields to its chains; pigp_potrf_lower's has the default priority
+    cudaStream_t bulk = nullptr;
+    std::vector<cudaEvent_t> pan, next;
+    cudaEvent_t done = nullptr;
+
+    int ensure(int panels) {
+        if (!bulk) {
+            int lo = 0, hi = 0;
+            if (low_priority) PIGP_CUDA(cudaDeviceGetStreamPriorityRange(&lo, &hi));
+            PIGP_CUDA(cudaStreamCreateWithPriority(&bulk, cudaStreamNonBlocking, lo));
+            PIGP_CUDA(cudaEventCreateWithFlags(&done, cudaEventDisableTiming));
+        }
+        while ((int)pan.size() < panels) {
+            cudaEvent_t a = nullptr, b = nullptr;
+            PIGP_CUDA(cudaEventCreateWithFlags(&a, cudaEventDisableTiming));
+            PIGP_CUDA(cudaEventCreateWithFlags(&b, cudaEventDisableTiming));
+            pan.push_back(a);
+            next.push_back(b);
+        }
+        return PIGP_OK;
+    }
+    void destroy() {
+        if (bulk) cudaStreamDestroy(bulk);
+        if (done) cudaEventDestroy(done);
+        for (cudaEvent_t e : pan) cudaEventDestroy(e);
+        for (cudaEvent_t e : next) cudaEventDestroy(e);
+    }
+};
+
 }  // namespace pigp
 
 using namespace pigp;
@@ -266,9 +300,7 @@ struct pigp_dsolver {
     cudaEvent_t ev_k = nullptr, ev_kd = nullptr;
     int k_done = 0;
     cudaStream_t se = nullptr;  // completes the inverse diagonal tiles (k_tile_inv) as soon as L_kk exists, off both chains
-    cudaStream_t sd = nullptr;                // bulk trailing updates of the panel schedule
-    std::vector<cudaEvent_t> ev_pan, ev_next; // per coarse panel: chain done / next panel's columns updated
-    cudaEvent_t ev_d = nullptr;
+    PanelSched panels{true};
 
     int f_diag(int k) const { return k; }
     int f_panel(int k, int src) const { return T + k * world + src; }
@@ -276,15 +308,14 @@ struct pigp_dsolver {
     int f_grad(int src) const { return T + T * world + world + src; }
     int f_bar(int src) const { return T + T * world + 2 * world + src; }
     template <class P> P* peer(int p, P* local) const { return reinterpret_cast<P*>(peer_slab[p] + (reinterpret_cast<char*>(local) - slab)); }
-    // first own tile >= a
-    int first_own(int a) const { return a + ((rank - a) % world + world) % world; }
-    int count_own(int a, int b) const { const int f = first_own(a); return f < b ? (b - f + world - 1) / world : 0; }
 };
 
 namespace pigp {
 FactorView factor_view(pigp_dsolver* s) {
     FactorView f{};
-    f.L = s->L; f.ld = s->ld; f.npad = s->npad; f.T = s->T; f.invd = s->invd;
+    f.L = s->L; f.ld = s->ld; f.T = s->T; f.invd = s->invd; f.info = s->info;
+    f.end = s->gy + 1;  // this rank's y tile rides through the TRSMs: L^-1 y comes out of the same launches
+    f.rank = s->rank; f.world = s->world;
     f.v = s->L + (int64_t)s->gy * TILE * s->ld;  // first row of the y tile: L^-1 y after the factorisation
     return f;
 }
@@ -293,7 +324,8 @@ FactorView factor_view(pigp_dsolver* s) {
 namespace {
 
 struct Ctx {
-    pigp_dsolver* s;
+    FactorView f;      // the matrix being factored
+    pigp_dsolver* s;   // everything else of the solver: only with grad or peers (null under pigp_potrf_lower)
     cudaStream_t st;   // chain stream
     cudaStream_t sb;   // side stream (Y = L^-T), used when grad is set
     cudaStream_t sc;   // publication stream
@@ -309,7 +341,7 @@ struct Ctx {
 
 Ctx make_ctx(pigp_dsolver* s, cudaStream_t st) {
     Ctx c{};
-    c.s = s; c.st = st;
+    c.f = factor_view(s); c.s = s; c.st = st;
     int k = 0;
     for (int p = 0; p < s->world; ++p)
         if (p != s->rank) { c.others[k] = p; c.pf.f[k] = s->peer(p, s->flags); ++k; }
@@ -373,12 +405,13 @@ PushSig make_sig(const Ctx& c, int idx) {
 }
 
 int leaf(const Ctx& c, int k) {
+    const FactorView& f = c.f;
     pigp_dsolver* s = c.s;
-    const int64_t ld = s->ld;
-    double* invk = s->invd + (int64_t)k * TILE * TILE;
-    double* Akk = s->L + (int64_t)k * TILE * ld + (int64_t)k * TILE;
-    const bool mine = (k % s->world == s->rank), multi = c.npeers > 0;
-    if (mine) PIGP_TRY(launch_potf2(Akk, ld, invk, s->info, k * TILE, c.st));
+    const int64_t ld = f.ld;
+    double* invk = f.invd + (int64_t)k * TILE * TILE;
+    double* Akk = f.L + (int64_t)k * TILE * ld + (int64_t)k * TILE;
+    const bool mine = (k % f.world == f.rank), multi = c.npeers > 0;
+    if (mine) PIGP_TRY(launch_potf2(Akk, ld, invk, f.info, k * TILE, c.st));
     if (c.grad || multi) PIGP_CUDA(cudaEventRecord(s->ev_diag[k], c.st));  // mine: inv(L_kk) is ready; else: the chain has reached leaf k
     if (mine && multi) {
         // publish inv(L_kk) and diag(L_kk) from the publication stream while the chain goes on with this rank's own TRSM
@@ -392,17 +425,17 @@ int leaf(const Ctx& c, int k) {
         PIGP_CUDA(cudaGetLastError());
     }
     {
-        // L_ik = A_ik inv(L_kk)^T for the own row tiles below (and the y tile)
-        const int first = s->first_own(k + 1), cnt = s->count_own(k + 1, s->gy + 1);
+        // L_ik = A_ik inv(L_kk)^T for the own row tiles below (and the rows below the matrix)
+        const int first = f.first_own(k + 1), cnt = f.count_own(k + 1, f.end);
         if (cnt > 0) {
             GemmDesc g{};
             g.M = cnt * TILE; g.N = TILE; g.K = TILE;
             g.alpha = 1.0; g.beta = 0.0;
-            double* Cb = s->L + (int64_t)first * TILE * ld + (int64_t)k * TILE;
+            double* Cb = f.L + (int64_t)first * TILE * ld + (int64_t)k * TILE;
             g.A = Cb; g.lda = ld; g.a_kcontig = 1;
             g.B = invk; g.ldb = TILE; g.b_kcontig = 1;
             g.C = Cb; g.ldc = ld;
-            g.gen = 1; g.m_ts = s->world; g.m_gt0 = first; g.n_gt0 = k; g.k_gt0 = k;
+            g.gen = 1; g.m_ts = f.world; g.m_gt0 = first; g.n_gt0 = k; g.k_gt0 = k;
             g.force_bn128 = 1;  // in place
             g.Lkk = Akk; g.ldl = ld;  // refined: needs L_kk itself next to its inverse (peers receive both)
             if (!mine) PIGP_TRY(set_wait_one(c, g, s->f_diag(k), c.st));
@@ -412,7 +445,7 @@ int leaf(const Ctx& c, int k) {
         if (multi) {
             // publish them (rows of the matrix proper; the y tile is private) and raise PANEL[k][rank] on every peer
             PIGP_CUDA(cudaStreamWaitEvent(c.sc, s->ev_upd[k], 0));
-            const int pcnt = s->count_own(k + 1, s->T);
+            const int pcnt = f.count_own(k + 1, f.T);
             ProfScope prof(PROF_MISC, c.sc);
             if (pcnt > 0) {
                 PeerBufs pb{};
@@ -435,7 +468,7 @@ int leaf(const Ctx& c, int k) {
         PIGP_TRY(launch_tile_inv(s->L, ld, s->invd, k, 1, 1, mine ? s->Y : nullptr, ld, c.se));
         PIGP_CUDA(cudaEventRecord(s->ev_inv[k], c.se));
         PIGP_CUDA(cudaStreamWaitEvent(c.sb, s->ev_inv[k], 0));
-        const int first = s->first_own(0), cnt = s->count_own(0, k);
+        const int first = f.first_own(0), cnt = f.count_own(0, k);
         if (cnt > 0) {
             GemmDesc g{};
             g.M = cnt * TILE; g.N = TILE; g.K = TILE;
@@ -471,32 +504,33 @@ int leaf(const Ctx& c, int k) {
 }
 
 int rec(const Ctx& c, int c0, int nt) {
-    pigp_dsolver* s = c.s;
     if (nt == 1) return leaf(c, c0);
-    const int64_t ld = s->ld;
+    const FactorView& f = c.f;
+    pigp_dsolver* s = c.s;
+    const int64_t ld = f.ld;
     const int n1 = nt / 2, n2 = nt - n1;
     PIGP_TRY(rec(c, c0, n1));
     const int k1 = c0 + n1 - 1;  // once every peer's PANEL[k1] flag is up, all rows of the panels [c0, c0 + n1) have arrived
     {
         // trailing update of the own row tiles: C[i, J2] -= L[i, K1] L[J2, K1]^T (lower part)
-        const int first = s->first_own(c0 + n1), cnt = s->count_own(c0 + n1, s->gy + 1);
+        const int first = f.first_own(c0 + n1), cnt = f.count_own(c0 + n1, f.end);
         if (cnt > 0) {
             GemmDesc g{};
             g.M = cnt * TILE; g.N = n2 * TILE; g.K = n1 * TILE;
             g.alpha = -1.0; g.beta = 1.0;
-            g.A = s->L + (int64_t)first * TILE * ld + (int64_t)c0 * TILE; g.lda = ld; g.a_kcontig = 1;
-            g.B = s->L + (int64_t)(c0 + n1) * TILE * ld + (int64_t)c0 * TILE; g.ldb = ld; g.b_kcontig = 1;
-            g.C = s->L + (int64_t)first * TILE * ld + (int64_t)(c0 + n1) * TILE; g.ldc = ld;
+            g.A = f.L + (int64_t)first * TILE * ld + (int64_t)c0 * TILE; g.lda = ld; g.a_kcontig = 1;
+            g.B = f.L + (int64_t)(c0 + n1) * TILE * ld + (int64_t)c0 * TILE; g.ldb = ld; g.b_kcontig = 1;
+            g.C = f.L + (int64_t)first * TILE * ld + (int64_t)(c0 + n1) * TILE; g.ldc = ld;
             g.lower_only = 1;
-            g.gen = 1; g.m_ts = s->world; g.m_gt0 = first; g.n_gt0 = c0 + n1; g.k_gt0 = c0;
-            PIGP_TRY(set_wait_all(c, g, s->f_panel(k1, 0), c.st));
+            g.gen = 1; g.m_ts = f.world; g.m_gt0 = first; g.n_gt0 = c0 + n1; g.k_gt0 = c0;
+            if (c.npeers > 0) PIGP_TRY(set_wait_all(c, g, s->f_panel(k1, 0), c.st));
             PIGP_TRY(launch_gemm(g, c.st));
         }
     }
     if (c.grad) {
         // Y[j, J2] -= sum_{k in K1, k >= j} Y[j, k] L[J2, k]^T for the own row tiles j < c0 + n1
         PIGP_CUDA(cudaStreamWaitEvent(c.sb, s->ev_upd[k1], 0));
-        const int first = s->first_own(0), cnt = s->count_own(0, c0 + n1);
+        const int first = f.first_own(0), cnt = f.count_own(0, c0 + n1);
         if (cnt > 0) {
             GemmDesc g{};
             g.M = cnt * TILE; g.N = n2 * TILE; g.K = n1 * TILE;
@@ -534,75 +568,61 @@ int rec(const Ctx& c, int c0, int nt) {
 // with the chain's work on panel p + 1.  The big trailing updates thereby leave the N/128-step dependency chain; the
 // L^-T products get the matching right-looking update V_p on the side stream.  Uses the existing kernels only.
 // Width: PIGP_LOOKAHEAD / pigp_set_lookahead(W >= 0) fix it (0 = plain recursion); unset (or a negative W) = automatic:
-// a single-rank NLL-only evaluation has no L^-T work on the side stream to fill the bubbles of the potf2 -> TRSM chain,
-// and the panel schedule measured 18 % / 13 % / 5 % faster there at N = 5018 / 10570 / 20000 (profiles/r02_lookahead.txt);
-// with the gradient requested the L^-T products fill most of those bubbles (a few per cent gain at mid sizes only), and
-// sharded runs keep the plain recursion.
+// a single-rank NLL-only evaluation (and pigp_potrf_lower) has no L^-T work on the side stream to fill the bubbles of the
+// potf2 -> TRSM chain, and the panel schedule measured 18 % / 13 % / 5 % faster there at N = 5018 / 10570 / 20000
+// (profiles/r02_lookahead.txt); with the gradient requested the L^-T products fill most of those bubbles (a few per cent
+// gain at mid sizes only), and sharded runs keep the plain recursion.
 static int g_lookahead = -2;  // -2: read PIGP_LOOKAHEAD once; -1: automatic; >= 0: fixed
-static int lookahead_width(const pigp_dsolver* s, bool grad) {
+static int lookahead_width(int T, int world, bool grad) {
     if (g_lookahead == -2) { const char* e = getenv("PIGP_LOOKAHEAD"); g_lookahead = e ? std::max(0, atoi(e)) : -1; }
     if (g_lookahead >= 0) return g_lookahead;
-    if (s->world != 1 || s->T < 12) return 0;
-    if (grad) return (s->T >= 16 && s->T < 32) ? 2 : (s->T >= 32 && s->T < 96) ? 4 : 0;  // -6 % at N = 2640, -4 % at 5018
-    return s->T < 64 ? 2 : s->T < 128 ? 4 : 16;
-}
-
-static int ensure_lookahead(pigp_dsolver* s) {
-    if (s->sd) return PIGP_OK;
-    int lo = 0, hi = 0;
-    PIGP_CUDA(cudaDeviceGetStreamPriorityRange(&lo, &hi));
-    PIGP_CUDA(cudaStreamCreateWithPriority(&s->sd, cudaStreamNonBlocking, lo));
-    PIGP_CUDA(cudaEventCreateWithFlags(&s->ev_d, cudaEventDisableTiming));
-    s->ev_pan.assign(s->T, nullptr);
-    s->ev_next.assign(s->T, nullptr);
-    for (int k = 0; k < s->T; ++k) {
-        PIGP_CUDA(cudaEventCreateWithFlags(&s->ev_pan[k], cudaEventDisableTiming));
-        PIGP_CUDA(cudaEventCreateWithFlags(&s->ev_next[k], cudaEventDisableTiming));
-    }
-    return PIGP_OK;
+    if (world != 1 || T < 12) return 0;
+    if (grad) return (T >= 16 && T < 32) ? 2 : (T >= 32 && T < 96) ? 4 : 0;  // -6 % at N = 2640, -4 % at 5018
+    return T < 64 ? 2 : T < 128 ? 4 : 16;
 }
 
 // C[i, J] -= L[i, Kp] L[J, Kp]^T for the own row tiles i >= jc0 (lower part), J = [jc0, jc1), Kp = [k0, k1)
 static int panel_update(const Ctx& c, int k0, int k1, int jc0, int jc1, cudaStream_t st) {
-    pigp_dsolver* s = c.s;
+    const FactorView& f = c.f;
     if (jc1 <= jc0) return PIGP_OK;
-    const int64_t ld = s->ld;
-    const int first = s->first_own(jc0), cnt = s->count_own(jc0, s->gy + 1);
+    const int64_t ld = f.ld;
+    const int first = f.first_own(jc0), cnt = f.count_own(jc0, f.end);
     if (cnt <= 0) return PIGP_OK;
     GemmDesc g{};
     g.M = cnt * TILE; g.N = (jc1 - jc0) * TILE; g.K = (k1 - k0) * TILE;
     g.alpha = -1.0; g.beta = 1.0;
-    g.A = s->L + (int64_t)first * TILE * ld + (int64_t)k0 * TILE; g.lda = ld; g.a_kcontig = 1;
-    g.B = s->L + (int64_t)jc0 * TILE * ld + (int64_t)k0 * TILE; g.ldb = ld; g.b_kcontig = 1;
-    g.C = s->L + (int64_t)first * TILE * ld + (int64_t)jc0 * TILE; g.ldc = ld;
+    g.A = f.L + (int64_t)first * TILE * ld + (int64_t)k0 * TILE; g.lda = ld; g.a_kcontig = 1;
+    g.B = f.L + (int64_t)jc0 * TILE * ld + (int64_t)k0 * TILE; g.ldb = ld; g.b_kcontig = 1;
+    g.C = f.L + (int64_t)first * TILE * ld + (int64_t)jc0 * TILE; g.ldc = ld;
     g.lower_only = 1;
-    g.gen = 1; g.m_ts = s->world; g.m_gt0 = first; g.n_gt0 = jc0; g.k_gt0 = k0;
+    g.gen = 1; g.m_ts = f.world; g.m_gt0 = first; g.n_gt0 = jc0; g.k_gt0 = k0;
     return launch_gemm(g, st);
 }
 
-static int chol_lookahead(const Ctx& c, int W) {
+static int chol_lookahead(const Ctx& c, int W, PanelSched& ps) {
+    const FactorView& f = c.f;
     pigp_dsolver* s = c.s;
-    PIGP_TRY(ensure_lookahead(s));
-    const int64_t ld = s->ld;
-    const int T = s->T;
+    const int64_t ld = f.ld;
+    const int T = f.T;
+    PIGP_TRY(ps.ensure((T + W - 1) / W));
     for (int j0 = 0, p = 0; j0 < T; j0 += W, ++p) {
         const int j1 = std::min(j0 + W, T);
         PIGP_TRY(rec(c, j0, j1 - j0));  // chain: panel p, all own rows below (and the intra-panel L^-T products on sb)
         if (j1 >= T) break;
-        PIGP_CUDA(cudaEventRecord(s->ev_pan[p], c.st));
+        PIGP_CUDA(cudaEventRecord(ps.pan[p], c.st));
         // bulk stream: panel p -> columns of panel p + 1 (the chain waits for this), then -> everything right of it
-        PIGP_CUDA(cudaStreamWaitEvent(s->sd, s->ev_pan[p], 0));
-        PIGP_TRY(wait_all(c, s->f_panel(j1 - 1, 0), s->sd));  // every peer's rows of the panel's columns have arrived
+        PIGP_CUDA(cudaStreamWaitEvent(ps.bulk, ps.pan[p], 0));
+        if (c.npeers > 0) PIGP_TRY(wait_all(c, s->f_panel(j1 - 1, 0), ps.bulk));  // every peer's rows of the panel have arrived
         const int jn = std::min(j1 + W, T);
-        PIGP_TRY(panel_update(c, j0, j1, j1, jn, s->sd));
-        PIGP_CUDA(cudaEventRecord(s->ev_next[p], s->sd));
-        PIGP_TRY(panel_update(c, j0, j1, jn, T, s->sd));
-        PIGP_CUDA(cudaStreamWaitEvent(c.st, s->ev_next[p], 0));
+        PIGP_TRY(panel_update(c, j0, j1, j1, jn, ps.bulk));
+        PIGP_CUDA(cudaEventRecord(ps.next[p], ps.bulk));
+        PIGP_TRY(panel_update(c, j0, j1, jn, T, ps.bulk));
+        PIGP_CUDA(cudaStreamWaitEvent(c.st, ps.next[p], 0));
         if (c.grad) {
             // V_p: Y[j, [j1, T)] -= sum_{k in panel p, k >= j} Y[j, k] L[[j1, T), k]^T for the own row tiles j < j1
-            PIGP_CUDA(cudaStreamWaitEvent(c.sb, s->ev_pan[p], 0));
+            PIGP_CUDA(cudaStreamWaitEvent(c.sb, ps.pan[p], 0));
             PIGP_TRY(wait_all(c, s->f_panel(j1 - 1, 0), c.sb));
-            const int first = s->first_own(0), cnt = s->count_own(0, j1);
+            const int first = f.first_own(0), cnt = f.count_own(0, j1);
             if (cnt > 0) {
                 GemmDesc g{};
                 g.M = cnt * TILE; g.N = (T - j1) * TILE; g.K = (j1 - j0) * TILE;
@@ -616,8 +636,8 @@ static int chol_lookahead(const Ctx& c, int W) {
             }
         }
     }
-    PIGP_CUDA(cudaEventRecord(s->ev_d, s->sd));
-    PIGP_CUDA(cudaStreamWaitEvent(c.st, s->ev_d, 0));
+    PIGP_CUDA(cudaEventRecord(ps.done, ps.bulk));
+    PIGP_CUDA(cudaStreamWaitEvent(c.st, ps.done, 0));
     return PIGP_OK;
 }
 
@@ -631,7 +651,36 @@ int preload_dist() {
     return PIGP_OK;
 }
 
+// pigp_potrf_lower's panel streams: one set per device, shared by the host threads that factor on it
+PanelSched g_panels[64];
+std::mutex g_panels_mutex;
+
 }  // namespace
+
+// pigp_potrf_lower: the solver's factorisation, on one rank, of the caller's buffer; its m_extra rows below the matrix
+// ride through the TRSMs and trailing updates as the solver's y tile does.
+int pigp::potrf_lower(double* A, int64_t ld, int64_t n, int64_t m_extra, double* invd, int32_t* info, cudaStream_t st) {
+    if (n <= 0 || n % TILE || m_extra % TILE || m_extra < 0 || ld % 2) {
+        set_error("pigp potrf: n and m_extra must be multiples of 128 and ld even");
+        return PIGP_EINVAL;
+    }
+    Ctx c{};
+    c.st = st;
+    c.f.L = A; c.f.ld = ld; c.f.invd = invd; c.f.info = info;
+    c.f.T = (int)(n / TILE); c.f.end = (int)((n + m_extra) / TILE);
+    c.f.rank = 0; c.f.world = 1;
+    const int W = lookahead_width(c.f.T, 1, false);
+    if (W > 0 && c.f.T > W) {
+        int dev = 0;
+        PIGP_CUDA(cudaGetDevice(&dev));
+        std::lock_guard<std::mutex> lock(g_panels_mutex);
+        PIGP_TRY(chol_lookahead(c, W, g_panels[dev & 63]));
+    } else {
+        PIGP_TRY(rec(c, 0, c.f.T));
+    }
+    // the factorisation leaves the diagonal 32-blocks of the inverse tiles; callers of this entry point get complete tiles
+    return launch_tile_inv(A, ld, invd, 0, 1, c.f.T, nullptr, 0, st, 1);
+}
 
 extern "C" {
 
@@ -645,10 +694,7 @@ void pigp_dsolver_destroy(pigp_dsolver* s) {
     if (s->sa) cudaStreamDestroy(s->sa);
     if (s->sb) cudaStreamDestroy(s->sb);
     if (s->sc) cudaStreamDestroy(s->sc);
-    if (s->sd) cudaStreamDestroy(s->sd);
-    if (s->ev_d) cudaEventDestroy(s->ev_d);
-    for (cudaEvent_t e : s->ev_pan) if (e) cudaEventDestroy(e);
-    for (cudaEvent_t e : s->ev_next) if (e) cudaEventDestroy(e);
+    s->panels.destroy();
     for (cudaEvent_t e : {s->ev_in, s->ev_bar, s->ev_b, s->ev_c, s->ev_out, s->ev_y0}) if (e) cudaEventDestroy(e);
     for (cudaEvent_t e : s->ev_diag) if (e) cudaEventDestroy(e);
     for (cudaEvent_t e : s->ev_upd) if (e) cudaEventDestroy(e);
@@ -674,7 +720,7 @@ int pigp_dsolver_create(pigp_plan* plan, int rank, int world, pigp_dsolver** out
     s->npad = round_up(s->n, TILE);
     s->ld = s->npad;
     s->T = (int)(s->npad / TILE);
-    s->gy = s->first_own(s->T);
+    s->gy = factor_view(s).first_own(s->T);  // the y tile: the first own tile past the matrix
     s->n_flags = s->T + s->T * world + 3 * world;
     const size_t l_bytes = sizeof(double) * (size_t)(s->T + world) * TILE * s->ld;
     // Y = L^-T is needed by the gradient only.  A single-rank solver (the handle behind pigp_solver: NLL-only and
@@ -744,6 +790,9 @@ int pigp_dsolver_create(pigp_plan* plan, int rank, int world, pigp_dsolver** out
             cuda_ok(cudaEventCreateWithFlags(&s->ev_inv[k], cudaEventDisableTiming), "cudaEventCreate");
         }
     }
+    // The zeroed flags, error flag and arrival counters must be in place before a peer signals into them, and cudaMemset
+    // is asynchronous to the host on the legacy stream, which does not order with any solver's non-blocking streams.
+    if (rc == PIGP_OK) cuda_ok(cudaStreamSynchronize(0), "cudaStreamSynchronize");
     if (rc != PIGP_OK) { pigp_dsolver_destroy(s); return rc; }
     s->connected = (world == 1);
     *out = s;
@@ -888,7 +937,7 @@ static int dsolver_enqueue(pigp_dsolver* s, const double* theta_dev, const doubl
     // every peer has finished reading what the previous call left in this rank's buffers
     PIGP_TRY(signal(c, s->f_bar(s->rank)));
     PIGP_TRY(wait_all(c, s->f_bar(0), st, barrier_timeout_ns()));
-    const int first = s->first_own(0), cnt = s->count_own(0, s->T);
+    const int first = c.f.first_own(0), cnt = c.f.count_own(0, s->T);
     if (c.grad && !s->Y) PIGP_CUDA(cudaMalloc(&s->Y, sizeof(double) * (size_t)s->npad * s->ld));
     if (c.grad) {
         PIGP_CUDA(cudaEventRecord(s->ev_bar, st));
@@ -917,8 +966,8 @@ static int dsolver_enqueue(pigp_dsolver* s, const double* theta_dev, const doubl
         count_launch();
     }
     PIGP_CUDA(cudaGetLastError());
-    const int law = lookahead_width(s, c.grad);
-    if (law > 0 && c.sb != st && s->T > law) PIGP_TRY(chol_lookahead(c, law));
+    const int law = lookahead_width(s->T, s->world, c.grad);
+    if (law > 0 && c.sb != st && s->T > law) PIGP_TRY(chol_lookahead(c, law, s->panels));
     else PIGP_TRY(rec(c, 0, s->T));
     if (c.npeers > 0) {
         // the diagonal of every L_kk (log-det) travels with the DIAG flags; a GEMM only waits for the flags it consumes
@@ -1008,12 +1057,14 @@ int pigp_dsolver_reset(pigp_dsolver* s) {
     PIGP_CUDA(cudaStreamSynchronize(s->sc));
     PIGP_CUDA(cudaStreamSynchronize(s->se));
     PIGP_CUDA(cudaStreamSynchronize(s->sk));
+    if (s->panels.bulk) PIGP_CUDA(cudaStreamSynchronize(s->panels.bulk));
     PIGP_CUDA(cudaMemset(s->err, 0, sizeof(int)));
     PIGP_CUDA(cudaMemset(s->sig_counter, 0, 2 * sizeof(unsigned int)));
     // the ranks' call counters may have drifted apart (a rank that never made the failed call): everybody restarts at
     // epoch 0 with clean flags.  The host-side barrier AFTER the resets keeps a fast rank's new flags from being erased.
     PIGP_CUDA(cudaMemset(s->flags, 0, sizeof(u64) * (size_t)s->n_flags));
     PIGP_CUDA(cudaMemset(s->gslots, 0, sizeof(double) * (size_t)s->world * MAX_THETA));
+    PIGP_CUDA(cudaStreamSynchronize(0));  // the memsets are complete when the host-side barrier is passed
     s->epoch = 0;
     s->broken = false;
     return PIGP_OK;

@@ -156,13 +156,20 @@ int launch_grad(const pigp_plan* p, const AsmTile* tiles, int64_t n_tiles, const
 // straddle a 128-row boundary
 void build_lower_tiles_owned(const pigp_plan* p, int rank, int world, std::vector<AsmTile>& out);
 
-// ---- what the posterior driver needs of a (world = 1) block-cyclic solver after an NLL evaluation (pigp_dist.cu)
+// ---- the matrix the tile Cholesky of pigp_dist.cu factors in place, and what the posterior driver reads of a (world = 1)
+// solver's factor after an NLL evaluation
 struct FactorView {
-    double* L;       // lower Cholesky factor, row-major, leading dimension ld (npad rows)
-    int64_t ld, npad;
-    int T;           // npad / 128
+    double* L;       // K -> lower Cholesky factor, row-major, leading dimension ld
+    int64_t ld;
+    int T;           // row tiles of the matrix proper (npad / 128)
+    int end;         // one past the last row tile that rides through the panel TRSMs and trailing updates (>= T)
     double* invd;    // T inverse diagonal tiles
-    double* v;       // L^-1 y (npad entries; zeros beyond n)
+    int32_t* info;   // first failing pivot (may be null)
+    int rank, world; // 128-row tile t belongs to rank t mod world
+    double* v;       // L^-1 y (npad entries; zeros beyond n): solver only
+    // first own tile >= a
+    int first_own(int a) const { return a + ((rank - a) % world + world) % world; }
+    int count_own(int a, int b) const { const int f = first_own(a); return f < b ? (b - f + world - 1) / world : 0; }
 };
 FactorView factor_view(pigp_dsolver* s);
 
@@ -211,13 +218,11 @@ int launch_potf2(double* A, int64_t ld, double* invd, int32_t* info, int base, c
 // write inv(L_cc)^T into the diagonal tile c of Y (row stride ldy)
 int launch_tile_inv(const double* L, int64_t ld, double* invd, int first, int stride, int count, double* Y, int64_t ldy, cudaStream_t st,
                     int zero_upper = 0);
+// pigp_potrf_lower (pigp_dist.cu: the solver's factorisation over the caller's buffer)
 int potrf_lower(double* A, int64_t ld, int64_t n, int64_t m_extra, double* invd, int32_t* info, cudaStream_t st);
 int potri_lower(const double* L, int64_t ld, int64_t n, const double* invd, double* W, double* X, cudaStream_t st);
 // out[0] = sum_{i<n} log A[i*ld+i]; out[1] = sum_{j<n} v[j]^2  (v = row `vrow` of A)
 int launch_logdet_quad(const double* A, int64_t ld, int64_t n, const double* v, double* out2, cudaStream_t st);
-// y[j] = sum_{i>=j} W[i*ld+j] x[i]   (W lower, n x n): alpha = W^T v
-// part: workspace of ceil(n/1024) * n doubles
-int launch_trmv_lower_t(const double* W, int64_t ld, int64_t n, const double* x, double* y, double* part, cudaStream_t st);
 // y[i] = sum_j A[i*ld+j] x[j], A (m x n) row-major
 int launch_gemv(const double* A, int64_t ld, int64_t m, int64_t n, const double* x, double* y, cudaStream_t st);
 

@@ -5,19 +5,20 @@ Which code runs depends on the tile count T = round_up(N, 128) / 128 (or n / 128
 
   regime                                          threshold (file:line)                       covered by
   ----------------------------------------------  ------------------------------------------  ---------------------------------
-  pigp_potrf_lower: recursion / panels W=2/4/16   pigp_dense.cu:1255 (breaks at 12, 64, 128)   test_potrf_potri_exact, T in
-                                                                                               POTRF_T (both sides of each break,
-                                                                                               odd T, short last panel)
-  block-TRSM slab height 8 / 16 / 32 rows         pigp_dense.cu:616-620 (1184 / 2368 rows)     same (panel heights up to 16.8k)
-  k_gemm BN 64 / 128, lower_only, remainder       pigp_dense.cu:691-724, PIGP_GEMM_BN           test_dgemm_*, test_knobs
-  small-tile GEMMs (solver launches)              pigp_dense.cu:691-709, PIGP_GEMM_SMALL        test_solver_regime, test_knobs
-  solver NLL + gradient: rec / W=2 / W=4 / rec    pigp_dist.cu:546 (16, 32, 96)                test_solver_regime, SOLVER_T
-  solver NLL only: rec / W=2 / 4 / 16             pigp_dist.cu:545-547 (12, 64, 128)           test_solver_regime (also width 0)
-  early K^-1 accumulation (one rank, 8..32)       pigp_dist.cu:883; late product :970-980      test_solver_regime (T 7/8, 32/33),
+  pigp_potrf_lower: recursion / panels W=2/4/16   pigp_dist.cu:579-581 (12, 64, 128)           test_potrf_potri_exact, T in
+                                                  (the solver's NLL-only rule)                 POTRF_T (both sides of each break,
+                                                                                               odd T, short last panel), T 17/65
+                                                                                               with pigp_set_lookahead(0)
+  block-TRSM slab height 8 / 16 / 32 rows         pigp_dense.cu:614-618 (1184 / 2368 rows)     same (panel heights up to 16.8k)
+  k_gemm BN 64 / 128, lower_only, remainder       pigp_dense.cu:689-722, PIGP_GEMM_BN           test_dgemm_*, test_knobs
+  small-tile GEMMs (solver launches)              pigp_dense.cu:689-707, PIGP_GEMM_SMALL        test_solver_regime, test_knobs
+  solver NLL + gradient: rec / W=2 / W=4 / rec    pigp_dist.cu:580 (16, 32, 96)                test_solver_regime, SOLVER_T
+  solver NLL only: rec / W=2 / 4 / 16             pigp_dist.cu:579-581 (12, 64, 128)           test_solver_regime (also width 0)
+  early K^-1 accumulation (one rank, 8..32)       pigp_dist.cu:929; late product :1016-1026    test_solver_regime (T 7/8, 32/33),
                                                                                                test_knobs (PIGP_EARLY_KINV=0)
   pigp_predict (factors through NLL only)         pigp_capi.cu:606                             test_solver_regime (M = 300)
   block-cyclic ranks                              pigp_dist.cu                                 test_ranks_at_33_tiles
-  reuse of one solver after a failed evaluation   pigp_dist.cu:887-912                         test_reuse_after_failure (T 4/16/40),
+  reuse of one solver after a failed evaluation   pigp_dist.cu:933-958                         test_reuse_after_failure (T 4/16/40),
                                                                                                test_adam_after_failure
 
 References: the exact-factor SPD family L0 = c I + R (R strictly lower in {-1, 0, 1}, c a power of two >= 4 sqrt(n)) has the
@@ -150,10 +151,12 @@ def _potrf_width(T):
     return 0 if T < 12 else 2 if T < 64 else 4 if T < 128 else 16
 
 
-@pytest.mark.parametrize("T", POTRF_T)
-def test_potrf_potri_exact(cuda_device, T):
+@pytest.mark.parametrize("T,lookahead", [pytest.param(T, -1, id=str(T)) for T in POTRF_T] +
+                         [pytest.param(T, 0, id=f"{T}-lookahead0") for T in (17, 65)])
+def test_potrf_potri_exact(cuda_device, T, lookahead):
     """pigp_potrf_lower / pigp_potri_lower against the exact factor, with poisoned inputs and workspaces, padded ld and
-    extra rows; every inverse diagonal tile checked."""
+    extra rows; every inverse diagonal tile checked.  lookahead = 0: pigp_set_lookahead(0), which steers pigp_potrf_lower
+    as it steers the solver, makes it take the plain recursion where the automatic width would take panels."""
     import torch
 
     L = _lib()
@@ -166,8 +169,12 @@ def test_potrf_potri_exact(cuda_device, T):
     L0, E, buf = _potrf_case(n, m_extra, ld, T, dev)
     invd = torch.full((T, TILE, TILE), float("nan"), dtype=torch.float64, device=dev)
     info = torch.full((1,), -7, dtype=torch.int32, device=dev)
-    L.check(lib.pigp_potrf_lower(buf.data_ptr(), ld, n, m_extra, invd.data_ptr(), info.data_ptr(), None))
-    torch.cuda.synchronize()
+    L.check(lib.pigp_set_lookahead(lookahead))
+    try:
+        L.check(lib.pigp_potrf_lower(buf.data_ptr(), ld, n, m_extra, invd.data_ptr(), info.data_ptr(), None))
+        torch.cuda.synchronize()
+    finally:
+        L.check(lib.pigp_set_lookahead(-1))
     assert int(info.item()) == 0
     _check_guards(buf, n, n + m_extra)
     e_L = relerr(buf[:n, :n].tril(), L0)
@@ -178,7 +185,8 @@ def test_potrf_potri_exact(cuda_device, T):
         Wk = invd[k]
         assert float(Wk.triu(1).abs().max()) == 0.0, f"inverse tile {k} is not zero above its diagonal"
         e_inv = max(e_inv, relerr(Wk, tri_inv(L0[k * TILE:(k + 1) * TILE, k * TILE:(k + 1) * TILE])))
-    print(f"\n[potrf T={T} W={_potrf_width(T)} m_extra={m_extra} ld={ld}] L {e_L:.1e} extra {e_E:.1e} "
+    W = _potrf_width(T) if lookahead < 0 else lookahead
+    print(f"\n[potrf T={T} W={W} m_extra={m_extra} ld={ld}] L {e_L:.1e} extra {e_E:.1e} "
           f"invd {e_inv:.1e} (bars 1e-13 / 1e-12 / 1e-12)")
     assert e_L <= 1e-13 and e_E <= 1e-12 and e_inv <= 1e-12
 
@@ -653,7 +661,7 @@ def knob_child_checks():
     dev = torch.device("cuda:0")
     test_dgemm_exact(dev, (2048, 2048, 2048), 1)
     test_dgemm_exact(dev, (4096, 1024, 512), 1)
-    test_potrf_potri_exact(dev, 17)
+    test_potrf_potri_exact(dev, 17, -1)
     pb = Problem(_n_for(16), dev)
     try:
         ref = pb.reference()
