@@ -42,10 +42,11 @@
 extern "C" {
 #endif
 
-#define PIGP_ABI_VERSION 2
+#define PIGP_ABI_VERSION 3
 #define PIGP_MAX_TERMS 8   /* monomials per block (3-D Kfzfz needs 7) */
 #define PIGP_MAX_GROUPS 4  /* hyper-parameter groups per model (ux, uy, uz, pp); a block may use all of them */
 #define PIGP_TILE 128      /* row/column padding unit of every factorisation buffer */
+#define PIGP_MAX_BATCH 65535 /* hyper-parameter vectors of one batched evaluation / starts of one multi-start Adam run */
 
 enum {
     PIGP_OK = 0,
@@ -161,6 +162,25 @@ int pigp_nll_grad(pigp_solver* s, const double* theta_dev, const double* y_dev, 
  * plan's coordinates; otherwise they are re-uploaded.  want_grad = 0 skips the gradient. */
 int pigp_nll_grad_host(pigp_solver* s, const double* theta_host, const double* pts_host, const double* y_host,
                        double eps, int want_grad, double* nll_host, double* grad_host, int32_t* info_host);
+/* pigp_nll_grad for n_theta hyper-parameter vectors that share the training points, y and eps, in one pass: every launch
+ * of the schedule is issued once, with one grid dimension more for the slot, so the launch count does not depend on
+ * n_theta.  Slot b reads thetas_dev[b][theta_len] and writes nll_dev[b], grad_dev[b][theta_len] (grad_dev NULL: NLL
+ * only) and info_dev[b] (may be NULL).  Each slot's results equal pigp_nll_grad / pigp_nll of its theta bit for bit; a
+ * non-positive pivot in one slot gives NaN and info for that slot only.  pigp_nll and pigp_nll_grad are the
+ * n_theta = 1 case.  Runs on the caller's stream and never synchronises, like pigp_nll_grad.
+ * PIGP_EINVAL before any launch for n_theta outside [1, PIGP_MAX_BATCH], a null pointer, or a sharded solver
+ * (world > 1).
+ * Memory: for n_theta > 1 the solver keeps a batch workspace, grown to the largest batch seen and freed by
+ * pigp_solver_destroy.  Per slot, with npad = N rounded up to 128: (npad + 128) * npad + npad * 128 doubles for L, its y
+ * row tile and the inverse diagonal tiles, plus npad^2 for L^-T when the gradient is asked for, plus npad^2 for K^-1 when
+ * 8 <= npad / 128 <= 32.  PIGP_ENOMEM when it cannot grow: nothing was launched, and the solver remains usable for single
+ * calls and smaller batches. */
+int pigp_nll_grad_batch(pigp_solver* s, int n_theta, const double* thetas_dev, const double* y_dev, double eps,
+                        double* nll_dev, double* grad_dev, int32_t* info_dev, void* stream);
+/* Host-buffer variant: thetas_host[n_theta][theta_len] -> nll_host[n_theta], grad_host[n_theta][theta_len] (want_grad),
+ * info_host[n_theta] (may be NULL). */
+int pigp_nll_grad_batch_host(pigp_solver* s, int n_theta, const double* thetas_host, const double* y_host, double eps,
+                             int want_grad, double* nll_host, double* grad_host, int32_t* info_host);
 
 /* predictingFunction_all (GP/gp.py:226-256, postGP :91-120).  mixed: rows = test points, cols = training points;
  * test: symmetric plan over the test points.  mu_dev[M] = K_ab K_bb^-1 y (mu_test is added by the caller);
@@ -195,6 +215,19 @@ int pigp_adam_host(pigp_solver* s, const double* theta0_host, const double* y_ho
                    double stop_eps, double ntraining, double ridge_alpha, int ridge_in_grad, const int32_t* fixed_host,
                    int check_every, double* theta_hist_host, double* loss_hist_host, double* norm_hist_host,
                    int32_t* n_done_host, int32_t* status_host);
+/* pigp_adam_host from n_start starting points theta0s_host[n_start][P] at once: one batched NLL + gradient evaluation
+ * (pigp_nll_grad_batch) and one update kernel (one warp per start) per iteration.  A start that has stopped (status != 0)
+ * is frozen: its later updates are no-ops.  The loop ends when every start has stopped or max_iter is reached.  Start b's
+ * outputs are theta_hist_host[b][max_iter + 1][P], loss_hist_host[b][max_iter + 1], norm_hist_host[b][max_iter] (the
+ * first n_done_host[b] + 1, n_done_host[b] + 1 and n_done_host[b] entries are written), n_done_host[b] and
+ * status_host[b], each equal bit for bit to pigp_adam_host from theta0s_host[b] alone.  pigp_adam_host is the
+ * n_start = 1 case, and like it runs on a sharded solver (every rank makes the same call); several starts need a
+ * world = 1 solver.  The loop runs on a stream of its own per solver.  PIGP_EINVAL for n_start outside
+ * [1, PIGP_MAX_BATCH], a null pointer, or n_start > 1 on a sharded solver. */
+int pigp_adam_batch_host(pigp_solver* s, int n_start, const double* theta0s_host, const double* y_host, double eps,
+                         int max_iter, double lr, double stop_eps, double ntraining, double ridge_alpha, int ridge_in_grad,
+                         const int32_t* fixed_host, int check_every, double* theta_hist_host, double* loss_hist_host,
+                         double* norm_hist_host, int32_t* n_done_host, int32_t* status_host);
 
 /* --- building blocks exposed for tests and benchmarks (device pointers, n multiple of PIGP_TILE) --- */
 /* In-place lower Cholesky of the leading n x n of A (row-major, ld), applying L^-T to the m_extra rows below it

@@ -245,6 +245,29 @@ class GPmodel:
             grad = full
         return nll, grad
 
+    def value_and_grad_many(self, thetas, r, delta_y, eps, want_grad=True):
+        """value_and_grad for every row of ``thetas`` -> (nll (B,), grad (B, P_caller) or None).  One pass of the
+        factorisation schedule evaluates all of them (Solver.nll_grad_batch_host); row b equals value_and_grad(thetas[b])
+        bit for bit.  A sharded model evaluates them one after another, so that every rank issues the same calls.  The
+        value_and_grad cache is left as it was."""
+        thetas = [np.asarray(t, dtype=np.float64).ravel() for t in thetas]
+        y = np.ascontiguousarray(np.asarray(delta_y, dtype=np.float64).ravel())
+        solver = self._solver_for(r)
+        if solver.world > 1:
+            cache = self._cache
+            out = [self.value_and_grad(t, r, y, eps, want_grad=want_grad) for t in thetas]
+            self._cache = cache
+            nll = np.array([o[0] for o in out])
+            return nll, (np.stack([o[1] for o in out]) if want_grad else None)
+        reduced = [self._reduce_theta(t) for t in thetas]
+        nll, grad, _info = solver.nll_grad_batch_host([th for th, _ in reduced], y, eps, want_grad=want_grad)
+        if grad is not None and any(idx is not None for _, idx in reduced):
+            full = np.zeros((len(thetas), thetas[0].size), dtype=np.float64)
+            for b, (_, idx) in enumerate(reduced):
+                full[b, slice(None) if idx is None else idx] = grad[b]
+            grad = full
+        return nll, grad
+
     def trainingFunction_all(self, theta, *args):
         """NLL (gp.py:213-224).  Once a gradient has been requested from this model (the explicit-derivative scripts call
         func(theta) and then dfunc(theta) every step, solver/optimizers.py:148-150), the gradient is evaluated along with
@@ -269,6 +292,21 @@ class GPmodel:
         self._cache = None
         return solver.adam_host(th, delta_y, eps, max_iter, lr, stop_eps, ntraining, ridge_alpha=ridge_alpha,
                                 ridge_in_grad=ridge_in_grad, fixed=fixed, check_every=check_every)
+
+    def adam_device_many(self, theta0s, r, delta_y, eps, max_iter, lr, stop_eps, ntraining, ridge_alpha=0.0,
+                         ridge_in_grad=True, fixed=None, check_every=16):
+        """adam_device from several starting points in one device loop (one batched evaluation per iteration) -> list of
+        adam_device's tuples, or None when a start carries entries held by the caller only, or the model is sharded."""
+        reduced = [self._reduce_theta(t) for t in theta0s]
+        if any(idx is not None for _, idx in reduced):
+            return None
+        solver = self._solver_for(r)
+        if solver.world > 1:
+            return None
+        self._cache = None
+        return solver.adam_batch_host([th for th, _ in reduced], delta_y, eps, max_iter, lr, stop_eps, ntraining,
+                                      ridge_alpha=ridge_alpha, ridge_in_grad=ridge_in_grad, fixed=fixed,
+                                      check_every=check_every)
 
     def d_logposterior(self, theta, *args):
         return self.d_trainingFunction_all(theta, *args) + 1.0  # gradient of the sum(theta) prior (gp.py:491-493)

@@ -11,7 +11,8 @@ MAX_GROUPS = 4
 TILE = 128
 LAYOUT_FULL, LAYOUT_LOWER = 0, 1
 IPC_HANDLE_BYTES = 64
-ABI_VERSION = 2
+ABI_VERSION = 3
+MAX_BATCH = 65535
 KERNEL_TYPES = {"se": 0, "mt52": 52, "mt72": 72, "mt92": 92}
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
@@ -64,6 +65,10 @@ _SIGNATURES = {
     "pigp_nll_grad": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_double, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "pigp_nll_grad_host": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_double, C.c_int, C.c_void_p,
                                      C.c_void_p, C.c_void_p]),
+    "pigp_nll_grad_batch": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_double, C.c_void_p, C.c_void_p,
+                                      C.c_void_p, C.c_void_p]),
+    "pigp_nll_grad_batch_host": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_double, C.c_int, C.c_void_p,
+                                           C.c_void_p, C.c_void_p]),
     "pigp_predict": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_double, C.c_void_p,
                                C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
     "pigp_predict_host": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_double, C.c_void_p,
@@ -73,6 +78,9 @@ _SIGNATURES = {
     "pigp_adam_host": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_double, C.c_int, C.c_double, C.c_double, C.c_double,
                                  C.c_double, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                  C.c_void_p]),
+    "pigp_adam_batch_host": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_double, C.c_int, C.c_double, C.c_double,
+                                       C.c_double, C.c_double, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
+                                       C.c_void_p, C.c_void_p]),
     "pigp_potrf_lower": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p]),
     "pigp_potri_lower": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "pigp_dgemm": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_double, C.c_void_p, C.c_int64, C.c_int, C.c_void_p, C.c_int64,

@@ -118,7 +118,8 @@ __global__ void k_rowsumsq_sub(const double* Vt, int64_t ld, int64_t m, int64_t 
     if (lane == 0) var[row] = kdiag[row] - s;
 }
 
-// ---- device-resident optimiser step (solver/optimizers.py:173-235): one warp, thread i owns hyper-parameter i
+// ---- device-resident optimiser step (solver/optimizers.py:173-235): one warp per start, thread i owns hyper-parameter i
+// (start b's arrays at + b times the size of one start's)
 struct AdamArgs {
     int P, max_iter;
     double lr, stop_eps, ntraining, ridge_alpha;
@@ -133,11 +134,19 @@ struct AdamArgs {
     double *theta_hist, *loss_hist, *norm_hist;
 };
 __global__ void k_adam_step(AdamArgs a) {
+    const int64_t b = blockIdx.x;
+    a.theta += b * a.P; a.m += b * a.P; a.v += b * a.P;
+    a.nll += b; a.grad += b * a.P; a.prev_loss += b;
+    a.istate += 4 * b;
+    a.theta_hist += b * (int64_t)(a.max_iter + 1) * a.P;
+    a.loss_hist += b * (int64_t)(a.max_iter + 1);
+    a.norm_hist += b * (int64_t)a.max_iter;
     const int i = threadIdx.x;
     const int t = a.istate[0];
     if (a.istate[2] != 0 || t >= a.max_iter) return;
     const bool on = i < a.P;
     const double th = on ? a.theta[i] : 0.0;
+    if (on && t == 0) a.theta_hist[i] = th;  // row 0 of the history: the starting point
     const double e2 = on ? exp(2.0 * th) : 0.0;
     double s_th = th, s_e2 = e2;
 #pragma unroll
@@ -235,6 +244,12 @@ struct pigp_solver {
     double* d_y = nullptr;
     double* d_res = nullptr;  // nll + grad
     double* h_res = nullptr;  // pinned
+    double* d_batch = nullptr;  // pigp_nll_grad_batch_host: thetas, nll, grad (grow-only)
+    int64_t batch_elems = 0;
+    int32_t* d_binfo = nullptr;
+    int64_t binfo_elems = 0;
+    // the device Adam loop runs on its own stream: ranks of a sharded solver that share a process must not share one
+    cudaStream_t adam_stream = nullptr;
 };
 
 static cudaStream_t as_stream(void* s) { return reinterpret_cast<cudaStream_t>(s); }
@@ -490,7 +505,8 @@ void pigp_solver_destroy(pigp_solver* s) {
     if (!s) return;
     pigp_dsolver_destroy(s->ds);
     cudaFree(s->info); cudaFree(s->V); cudaFree(s->T); cudaFree(s->kdiag); cudaFree(s->d_mu); cudaFree(s->d_cov);
-    cudaFree(s->d_theta); cudaFree(s->d_y); cudaFree(s->d_res);
+    cudaFree(s->d_theta); cudaFree(s->d_y); cudaFree(s->d_res); cudaFree(s->d_batch); cudaFree(s->d_binfo);
+    if (s->adam_stream) cudaStreamDestroy(s->adam_stream);
     if (s->h_res) cudaFreeHost(s->h_res);
     delete s;
 }
@@ -517,6 +533,7 @@ int pigp_solver_create_dist(pigp_plan* plan, int rank, int world, pigp_solver** 
     cuda_ok(cudaMalloc(&s->d_y, sizeof(double) * s->n), "cudaMalloc y");
     cuda_ok(cudaMalloc(&s->d_res, sizeof(double) * (1 + MAX_THETA)), "cudaMalloc res");
     cuda_ok(cudaMallocHost(&s->h_res, sizeof(double) * (2 + 2 * MAX_THETA) + sizeof(double) * s->n), "cudaMallocHost res");
+    cuda_ok(cudaStreamCreateWithFlags(&s->adam_stream, cudaStreamNonBlocking), "cudaStreamCreate adam");
     if (rc != PIGP_OK) { pigp_solver_destroy(s); return rc; }
     *out = s;
     return PIGP_OK;
@@ -587,6 +604,36 @@ int pigp_nll_grad_host(pigp_solver* s, const double* theta_host, const double* p
     *nll_host = s->h_res[0];
     if (want_grad) std::memcpy(grad_host, s->h_res + 1, sizeof(double) * P);
     if (info_host) *info_host = *h_info;
+    return PIGP_OK;
+}
+
+int pigp_nll_grad_batch(pigp_solver* s, int n_theta, const double* thetas_dev, const double* y_dev, double eps, double* nll_dev,
+                        double* grad_dev, int32_t* info_dev, void* stream) {
+    if (!s || !thetas_dev || !y_dev || !nll_dev) { set_error("pigp_nll_grad_batch: null argument"); return PIGP_EINVAL; }
+    if (n_theta < 1 || n_theta > PIGP_MAX_BATCH) { set_error("pigp_nll_grad_batch: n_theta must be in [1, 65535]"); return PIGP_EINVAL; }
+    if (s->world != 1) { set_error("pigp_nll_grad_batch: sharded solvers (world > 1) evaluate one theta at a time"); return PIGP_EINVAL; }
+    PIGP_TRY(use_device(s->plan));
+    return dsolver_nll_grad_batch(s->ds, n_theta, thetas_dev, y_dev, eps, nll_dev, grad_dev, info_dev, stream);
+}
+
+int pigp_nll_grad_batch_host(pigp_solver* s, int n_theta, const double* thetas_host, const double* y_host, double eps,
+                             int want_grad, double* nll_host, double* grad_host, int32_t* info_host) {
+    if (!s || !thetas_host || !y_host || !nll_host || (want_grad && !grad_host)) { set_error("pigp_nll_grad_batch_host: null argument"); return PIGP_EINVAL; }
+    if (n_theta < 1 || n_theta > PIGP_MAX_BATCH) { set_error("pigp_nll_grad_batch_host: n_theta must be in [1, 65535]"); return PIGP_EINVAL; }
+    if (s->world != 1) { set_error("pigp_nll_grad_batch_host: sharded solvers (world > 1) evaluate one theta at a time"); return PIGP_EINVAL; }
+    PIGP_TRY(use_device(s->plan));
+    const int64_t P = s->plan->theta_len, nb = n_theta;
+    PIGP_TRY(grow(&s->d_batch, &s->batch_elems, nb * (2 * P + 1)));
+    PIGP_TRY(grow(&s->d_binfo, &s->binfo_elems, nb));
+    double* th = s->d_batch;
+    double* nll = th + nb * P;
+    double* grad = nll + nb;
+    PIGP_CUDA(cudaMemcpy(th, thetas_host, sizeof(double) * nb * P, cudaMemcpyHostToDevice));
+    PIGP_CUDA(cudaMemcpy(s->d_y, y_host, sizeof(double) * s->n, cudaMemcpyHostToDevice));
+    PIGP_TRY(pigp_nll_grad_batch(s, n_theta, th, s->d_y, eps, nll, want_grad ? grad : nullptr, s->d_binfo, nullptr));
+    PIGP_CUDA(cudaMemcpy(nll_host, nll, sizeof(double) * nb, cudaMemcpyDeviceToHost));
+    if (want_grad) PIGP_CUDA(cudaMemcpy(grad_host, grad, sizeof(double) * nb * P, cudaMemcpyDeviceToHost));
+    if (info_host) PIGP_CUDA(cudaMemcpy(info_host, s->d_binfo, sizeof(int32_t) * nb, cudaMemcpyDeviceToHost));
     return PIGP_OK;
 }
 
@@ -679,63 +726,88 @@ int pigp_adam_host(pigp_solver* s, const double* theta0_host, const double* y_ho
                    double stop_eps, double ntraining, double ridge_alpha, int ridge_in_grad, const int32_t* fixed_host,
                    int check_every, double* theta_hist_host, double* loss_hist_host, double* norm_hist_host,
                    int32_t* n_done_host, int32_t* status_host) {
-    if (!s || !theta0_host || !y_host || !theta_hist_host || !loss_hist_host || !norm_hist_host || !n_done_host || !status_host ||
-        max_iter < 1 || !(ntraining > 0.0)) {
-        set_error("pigp_adam_host: bad argument");
+    return pigp_adam_batch_host(s, 1, theta0_host, y_host, eps, max_iter, lr, stop_eps, ntraining, ridge_alpha, ridge_in_grad,
+                                fixed_host, check_every, theta_hist_host, loss_hist_host, norm_hist_host, n_done_host, status_host);
+}
+
+int pigp_adam_batch_host(pigp_solver* s, int n_start, const double* theta0s_host, const double* y_host, double eps, int max_iter,
+                         double lr, double stop_eps, double ntraining, double ridge_alpha, int ridge_in_grad,
+                         const int32_t* fixed_host, int check_every, double* theta_hist_host, double* loss_hist_host,
+                         double* norm_hist_host, int32_t* n_done_host, int32_t* status_host) {
+    if (!s || !theta0s_host || !y_host || !theta_hist_host || !loss_hist_host || !norm_hist_host || !n_done_host || !status_host ||
+        max_iter < 1 || !(ntraining > 0.0) || n_start < 1 || n_start > PIGP_MAX_BATCH || (n_start > 1 && s->world != 1)) {
+        set_error("pigp_adam_host: bad argument (null pointer, max_iter < 1, ntraining <= 0, n_start outside [1, 65535], or "
+                  "several starts on a sharded solver)");
         return PIGP_EINVAL;
     }
     PIGP_TRY(use_device(s->plan));
     const int P = s->plan->theta_len;
+    const int64_t nb = n_start, H = (int64_t)(max_iter + 1) * P;
     if (check_every < 1) check_every = 16;
-    // workspace: [theta | m | v | nll | grad | prev_loss] doubles, histories, integer state, mask
-    const size_t n_d = (size_t)4 * MAX_THETA + 2 + (size_t)(max_iter + 1) * P + (size_t)(max_iter + 1) + (size_t)max_iter;
+    // workspace, one array of n_start entries each: theta, m, v, grad [P], nll, prev_loss, theta / loss / norm histories;
+    // integer state [4] per start, then the mask
+    const size_t n_d = (size_t)nb * (4 * P + 2 + H + (max_iter + 1) + max_iter);
     double* ws = nullptr;
     int32_t* iws = nullptr;
-    PIGP_CUDA(cudaMalloc(&ws, sizeof(double) * n_d));
-    if (cudaMalloc(&iws, sizeof(int32_t) * (4 + MAX_THETA)) != cudaSuccess) { cudaFree(ws); set_error("pigp_adam_host: out of memory"); return PIGP_ENOMEM; }
+    if (cudaMalloc(&ws, sizeof(double) * n_d) != cudaSuccess) { cudaGetLastError(); set_error("pigp_adam_host: out of memory"); return PIGP_ENOMEM; }
+    if (cudaMalloc(&iws, sizeof(int32_t) * (4 * nb + MAX_THETA)) != cudaSuccess) { cudaGetLastError(); cudaFree(ws); set_error("pigp_adam_host: out of memory"); return PIGP_ENOMEM; }
     int rc = PIGP_OK;
     auto ck = [&](cudaError_t e) { if (e != cudaSuccess && rc == PIGP_OK) { set_error(std::string("pigp_adam_host: ") + cudaGetErrorString(e)); rc = PIGP_ECUDA; } };
-    ck(cudaMemset(ws, 0, sizeof(double) * n_d));
-    ck(cudaMemset(iws, 0, sizeof(int32_t) * (4 + MAX_THETA)));
+    cudaStream_t st = s->adam_stream;
+    ck(cudaMemsetAsync(ws, 0, sizeof(double) * n_d, st));
+    ck(cudaMemsetAsync(iws, 0, sizeof(int32_t) * (4 * nb + MAX_THETA), st));
     AdamArgs a{};
     a.P = P; a.max_iter = max_iter; a.lr = lr; a.stop_eps = stop_eps; a.ntraining = ntraining;
     a.ridge_alpha = ridge_alpha; a.ridge_in_grad = ridge_in_grad;
-    a.theta = ws; a.m = ws + MAX_THETA; a.v = ws + 2 * MAX_THETA;
-    double* d_nll = ws + 3 * MAX_THETA;           // nll followed by the gradient
-    a.nll = d_nll; a.grad = d_nll + 1;
-    a.prev_loss = ws + 4 * MAX_THETA + 1;
-    a.theta_hist = ws + 4 * MAX_THETA + 2;
-    a.loss_hist = a.theta_hist + (size_t)(max_iter + 1) * P;
-    a.norm_hist = a.loss_hist + (max_iter + 1);
+    a.theta = ws; a.m = ws + nb * P; a.v = ws + 2 * nb * P;
+    double* d_grad = ws + 3 * nb * P;
+    double* d_nll = ws + 4 * nb * P;
+    a.nll = d_nll; a.grad = d_grad;
+    a.prev_loss = d_nll + nb;
+    a.theta_hist = a.prev_loss + nb;
+    a.loss_hist = a.theta_hist + nb * H;
+    a.norm_hist = a.loss_hist + nb * (max_iter + 1);
     a.istate = iws;
-    a.fixed = fixed_host ? iws + 4 : nullptr;
-    ck(cudaMemcpy(a.theta, theta0_host, sizeof(double) * P, cudaMemcpyHostToDevice));
-    ck(cudaMemcpy(a.theta_hist, theta0_host, sizeof(double) * P, cudaMemcpyHostToDevice));
-    ck(cudaMemcpy(s->d_y, y_host, sizeof(double) * s->n, cudaMemcpyHostToDevice));
-    if (fixed_host) ck(cudaMemcpy(iws + 4, fixed_host, sizeof(int32_t) * P, cudaMemcpyHostToDevice));
-    int32_t ist[4] = {0, 0, 0, 0};
+    a.fixed = fixed_host ? iws + 4 * nb : nullptr;
+    ck(cudaMemcpyAsync(a.theta, theta0s_host, sizeof(double) * nb * P, cudaMemcpyHostToDevice, st));
+    ck(cudaMemcpyAsync(s->d_y, y_host, sizeof(double) * s->n, cudaMemcpyHostToDevice, st));
+    if (fixed_host) ck(cudaMemcpyAsync(iws + 4 * nb, fixed_host, sizeof(int32_t) * P, cudaMemcpyHostToDevice, st));
+    std::vector<int32_t> ist((size_t)4 * nb, 0);
+    auto running = [&]() {
+        for (int64_t b = 0; b < nb; ++b)
+            if (ist[4 * b + 2] == 0) return true;
+        return false;
+    };
     // theta never leaves the device: evaluation and update are enqueued back to back, the host looks at the state only
-    // every check_every iterations (a plateau found in between leaves the remaining queued updates as no-ops)
-    for (int it = 0; it < max_iter && rc == PIGP_OK && ist[2] == 0; it += check_every) {
+    // every check_every iterations (a start that stopped in between leaves its remaining queued updates as no-ops)
+    for (int it = 0; it < max_iter && rc == PIGP_OK && running(); it += check_every) {
         const int nk = std::min(check_every, max_iter - it);
         for (int k = 0; k < nk && rc == PIGP_OK; ++k) {
-            rc = pigp_dsolver_nll_grad(s->ds, a.theta, s->d_y, eps, d_nll, d_nll + 1, s->info, nullptr);
+            // one start: the single-theta evaluation, which sharded solvers run too
+            rc = nb == 1 ? pigp_dsolver_nll_grad(s->ds, a.theta, s->d_y, eps, d_nll, d_grad, s->info, st)
+                         : pigp_nll_grad_batch(s, n_start, a.theta, s->d_y, eps, d_nll, d_grad, nullptr, st);
             if (rc == PIGP_OK) {
-                k_adam_step<<<1, 32>>>(a);
+                k_adam_step<<<(unsigned)nb, 32, 0, st>>>(a);
                 count_launch();
                 ck(cudaGetLastError());
             }
         }
-        ck(cudaMemcpy(ist, iws, sizeof(ist), cudaMemcpyDeviceToHost));
+        ck(cudaMemcpyAsync(ist.data(), iws, sizeof(int32_t) * 4 * nb, cudaMemcpyDeviceToHost, st));
+        ck(cudaStreamSynchronize(st));
     }
-    if (rc == PIGP_OK) {
-        const int done = ist[3];
-        ck(cudaMemcpy(theta_hist_host, a.theta_hist, sizeof(double) * (size_t)(done + 1) * P, cudaMemcpyDeviceToHost));
-        ck(cudaMemcpy(loss_hist_host, a.loss_hist, sizeof(double) * (size_t)(done + 1), cudaMemcpyDeviceToHost));
-        if (done > 0) ck(cudaMemcpy(norm_hist_host, a.norm_hist, sizeof(double) * (size_t)done, cudaMemcpyDeviceToHost));
-        *n_done_host = done;
-        *status_host = ist[2];
+    for (int64_t b = 0; b < nb && rc == PIGP_OK; ++b) {
+        const int done = ist[4 * b + 3];
+        ck(cudaMemcpyAsync(theta_hist_host + b * H, a.theta_hist + b * H, sizeof(double) * (size_t)(done + 1) * P,
+                           cudaMemcpyDeviceToHost, st));
+        ck(cudaMemcpyAsync(loss_hist_host + b * (max_iter + 1), a.loss_hist + b * (max_iter + 1), sizeof(double) * (size_t)(done + 1),
+                           cudaMemcpyDeviceToHost, st));
+        if (done > 0)
+            ck(cudaMemcpyAsync(norm_hist_host + b * max_iter, a.norm_hist + b * max_iter, sizeof(double) * (size_t)done,
+                               cudaMemcpyDeviceToHost, st));
+        n_done_host[b] = done;
+        status_host[b] = ist[4 * b + 2];
     }
+    ck(cudaStreamSynchronize(st));
     cudaFree(ws);
     cudaFree(iws);
     return rc;

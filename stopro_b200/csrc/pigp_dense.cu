@@ -105,6 +105,15 @@ __device__ __forceinline__ void load_frags(double2* frag, const double* sm, int 
     }
 }
 
+// the slot's operands (batched launches: once, at kernel entry)
+__device__ __forceinline__ void slot_ptrs(GemmDesc& g) {
+    const int64_t b = blockIdx.y;
+    g.A += b * g.sa;
+    g.B += b * g.sb;
+    g.C += b * g.sc;
+    if (g.Lkk) g.Lkk += b * g.sl;
+}
+
 // Bounded spin on epoch flags written by peers (st.release.sys); see pigp_dist.cu.
 __device__ __forceinline__ void wait_flags(const GemmDesc& g, int tid) {
     if (g.wait_count <= 0) return;
@@ -125,7 +134,9 @@ __device__ __forceinline__ void wait_flags(const GemmDesc& g, int tid) {
 
 // BN_ = 128: 8 warps, one CTA per SM.  BN_ = 64: 4 warps, two CTAs per SM (independent barriers: while one CTA waits at its
 // barrier or on shared-memory loads, the other keeps the FP64 tensor pipe busy).
-template <bool AKC, bool BKC, int BN_, int STAGES_>
+// BATCH: the launch covers g.nb slots (grid dimension y).  The kernels that can be batched are instantiated twice: the
+// single-slot instantiation is the kernel as it was before batching existed, instruction for instruction.
+template <bool AKC, bool BKC, int BN_, int STAGES_, bool BATCH>
 __global__ void __launch_bounds__(BN_ * 2, 128 / BN_) k_gemm(GemmDesc g) {
     constexpr int THREADS = BN_ * 2;
     constexpr int OPA = opd(BM), OPB = opd(BN_), STG = OPA + OPB;
@@ -163,6 +174,7 @@ __global__ void __launch_bounds__(BN_ * 2, 128 / BN_) k_gemm(GemmDesc g) {
     else if (g.kmode == 2) kt_end = min(kt_end, (gm - g.k_gt0 + 1) * (BM / BK));
     if (kt_end <= kt_begin && g.beta == 1.0) return;  // nothing to add
     wait_flags(g, tid);
+    if (BATCH) slot_ptrs(g);
 
     double acc[8][4][2];
 #pragma unroll
@@ -253,18 +265,23 @@ __global__ void __launch_bounds__(BN_ * 2, 128 / BN_) k_gemm(GemmDesc g) {
     }
 }
 
+template <int BN_, int STAGES_, bool BATCH>
+static int gemm_attrs_b() {
+    constexpr int SMEM = gemm_smem(BN_, STAGES_);
+    PIGP_CUDA(cudaFuncSetAttribute(k_gemm<true, true, BN_, STAGES_, BATCH>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM));
+    PIGP_CUDA(cudaFuncSetAttribute(k_gemm<true, false, BN_, STAGES_, BATCH>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM));
+    PIGP_CUDA(cudaFuncSetAttribute(k_gemm<false, true, BN_, STAGES_, BATCH>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM));
+    PIGP_CUDA(cudaFuncSetAttribute(k_gemm<false, false, BN_, STAGES_, BATCH>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM));
+    PIGP_PRELOAD((k_gemm<true, true, BN_, STAGES_, BATCH>));
+    PIGP_PRELOAD((k_gemm<true, false, BN_, STAGES_, BATCH>));
+    PIGP_PRELOAD((k_gemm<false, true, BN_, STAGES_, BATCH>));
+    PIGP_PRELOAD((k_gemm<false, false, BN_, STAGES_, BATCH>));
+    return PIGP_OK;
+}
 template <int BN_, int STAGES_>
 static int gemm_attrs() {
-    constexpr int SMEM = gemm_smem(BN_, STAGES_);
-    PIGP_CUDA(cudaFuncSetAttribute(k_gemm<true, true, BN_, STAGES_>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM));
-    PIGP_CUDA(cudaFuncSetAttribute(k_gemm<true, false, BN_, STAGES_>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM));
-    PIGP_CUDA(cudaFuncSetAttribute(k_gemm<false, true, BN_, STAGES_>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM));
-    PIGP_CUDA(cudaFuncSetAttribute(k_gemm<false, false, BN_, STAGES_>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM));
-    PIGP_PRELOAD((k_gemm<true, true, BN_, STAGES_>));
-    PIGP_PRELOAD((k_gemm<true, false, BN_, STAGES_>));
-    PIGP_PRELOAD((k_gemm<false, true, BN_, STAGES_>));
-    PIGP_PRELOAD((k_gemm<false, false, BN_, STAGES_>));
-    return PIGP_OK;
+    PIGP_TRY((gemm_attrs_b<BN_, STAGES_, false>()));
+    return gemm_attrs_b<BN_, STAGES_, true>();
 }
 
 // ----------------------------------------------------------------------------------------------- small-tile GEMM
@@ -272,7 +289,7 @@ static int gemm_attrs() {
 // the latency-bound launches of the factorisation (the K = 128 TRSM by the inverse diagonal tile, the low levels of
 // the trailing updates): 4-8 x more CTAs than 128 x 64 tiles, so that a 26-row-tile panel still covers the GPU.
 // BN_ = 128 with N = 128 is safe in place (C aliasing A): a CTA reads all 128 columns of its rows before it writes.
-template <int BM_, int BN_, int STAGES_>
+template <int BM_, int BN_, int STAGES_, bool BATCH>
 __global__ void __launch_bounds__(BN_ * 2) k_gemm_s(GemmDesc g) {
     constexpr int THREADS = BN_ * 2;
     constexpr int MI = BM_ / 16;  // 8-row MMA tiles per warp (2 warps along M)
@@ -294,6 +311,7 @@ __global__ void __launch_bounds__(BN_ * 2) k_gemm_s(GemmDesc g) {
     if (g.kmode == 1) kt_begin = max(0, gm - g.k_gt0) * (BM / BK);
     if (kt_end <= kt_begin && g.beta == 1.0) return;
     wait_flags(g, tid);
+    if (BATCH) slot_ptrs(g);
 
     // C -= A B^T (the trailing updates on the latency-bound chain): the accumulators start from -C, fetched while the first
     // operand tiles are still in flight, instead of a read-modify-write of C after the last MMA
@@ -410,7 +428,8 @@ static int launch_gemm_small(const GemmDesc& d, cudaStream_t st) {
     int dev = 0;
     PIGP_CUDA(cudaGetDevice(&dev));
     if (!attr_done[dev & 63]) {
-        PIGP_CUDA(cudaFuncSetAttribute(k_gemm_s<BM_, BN_, STAGES_>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM));
+        PIGP_CUDA(cudaFuncSetAttribute(k_gemm_s<BM_, BN_, STAGES_, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM));
+        PIGP_CUDA(cudaFuncSetAttribute(k_gemm_s<BM_, BN_, STAGES_, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM));
         attr_done[dev & 63] = true;
     }
     const int64_t ctas = (int64_t)(d.M / BM_) * (d.N / BN_);
@@ -425,8 +444,10 @@ static int launch_gemm_small(const GemmDesc& d, cudaStream_t st) {
         }
         prof_note(d.M, d.N, d.K, 100 + d.kmode * 10 + d.lower_only);
     }
-    ProfScope prof(PROF_GEMM, st, flops);
-    k_gemm_s<BM_, BN_, STAGES_><<<(unsigned)ctas, BN_ * 2, SMEM, st>>>(d);
+    ProfScope prof(PROF_GEMM, st, flops * d.nb);
+    const dim3 grid((unsigned)ctas, (unsigned)d.nb);
+    if (d.nb > 1) k_gemm_s<BM_, BN_, STAGES_, true><<<grid, BN_ * 2, SMEM, st>>>(d);
+    else k_gemm_s<BM_, BN_, STAGES_, false><<<grid, BN_ * 2, SMEM, st>>>(d);
     count_launch();
     return PIGP_OK;
 }
@@ -464,7 +485,7 @@ __device__ __forceinline__ void tile_mma(double (&d)[2], double (&e)[2], const d
     e[0] += h[0]; e[1] += h[1];
 }
 
-template <int TR_BM>
+template <int TR_BM, bool BATCH>
 __global__ void __launch_bounds__(256) k_trsm_blk(GemmDesc g) {
     constexpr int N_TILES = TR_BM / 8 * 4;                 // 8 x 8 tiles of one TR_BM x 32 block
     constexpr int TPW = N_TILES >= 8 ? N_TILES / 8 : 1;    // tiles per warp
@@ -480,6 +501,7 @@ __global__ void __launch_bounds__(256) k_trsm_blk(GemmDesc g) {
     const int tm = blockIdx.x;
     const int64_t m0 = (int64_t)(tm / SUB) * g.m_ts * BM + (tm % SUB) * TR_BM;
     wait_flags(g, tid);
+    if (BATCH) slot_ptrs(g);
     // one group of asynchronous copies per column block: what step jb needs (its 32 columns of the slab, row jb of the
     // blocks of Lkk, W_jb) arrives while steps 0 .. jb - 1 compute.  Thread (lr, lch) copies 16 bytes of rows lr and
     // lr + 16 of every 32 x 32 block: all offsets are compile-time multiples of the row strides (the issue of these ~30
@@ -595,7 +617,8 @@ static int launch_trsm_blk_t(const GemmDesc& d, cudaStream_t st) {
     int dev = 0;
     PIGP_CUDA(cudaGetDevice(&dev));
     if (!attr_done[dev & 63]) {
-        PIGP_CUDA(cudaFuncSetAttribute(k_trsm_blk<TR_BM>, cudaFuncAttributeMaxDynamicSharedMemorySize, tb_smem(TR_BM)));
+        PIGP_CUDA(cudaFuncSetAttribute(k_trsm_blk<TR_BM, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, tb_smem(TR_BM)));
+        PIGP_CUDA(cudaFuncSetAttribute(k_trsm_blk<TR_BM, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, tb_smem(TR_BM)));
         attr_done[dev & 63] = true;
     }
     double flops = 0.0;
@@ -603,8 +626,10 @@ static int launch_trsm_blk_t(const GemmDesc& d, cudaStream_t st) {
         flops = 18.0 * 2.0 * d.M * 32.0 * 32.0;
         prof_note(d.M, d.N, d.K, 200);
     }
-    ProfScope prof(PROF_GEMM, st, flops);
-    k_trsm_blk<TR_BM><<<(unsigned)(d.M / TR_BM), 256, tb_smem(TR_BM), st>>>(d);
+    ProfScope prof(PROF_GEMM, st, flops * d.nb);
+    const dim3 grid((unsigned)(d.M / TR_BM), (unsigned)d.nb);
+    if (d.nb > 1) k_trsm_blk<TR_BM, true><<<grid, 256, tb_smem(TR_BM), st>>>(d);
+    else k_trsm_blk<TR_BM, false><<<grid, 256, tb_smem(TR_BM), st>>>(d);
     count_launch();
     return PIGP_OK;
 }
@@ -634,7 +659,7 @@ static int launch_gemm_cfg(const GemmDesc& d, cudaStream_t st) {
     const int dmt = tri ? d.N / BM : d.M / BM, dnt_e = d.N / BM;  // in 128-element units
     const int smt = (dmt + SUPER - 1) / SUPER, snt = (dnt_e + SUPER - 1) / SUPER;
     const int64_t supers = tri ? (int64_t)smt * (smt + 1) / 2 : (int64_t)smt * snt;
-    const dim3 grid((unsigned)(supers * SUPER * SUPER * (BM / BN_))), block(BN_ * 2);
+    const dim3 grid((unsigned)(supers * SUPER * SUPER * (BM / BN_)), (unsigned)d.nb), block(BN_ * 2);
     double flops = 0.0;
     if (g_prof_on) {  // flops executed at 128-tile granularity
         const int kt = d.K / BK, per = BM / BK;
@@ -648,11 +673,18 @@ static int launch_gemm_cfg(const GemmDesc& d, cudaStream_t st) {
         }
         prof_note(tri ? d.N : d.M, d.N, d.K, d.kmode * 10 + d.lower_only);
     }
-    ProfScope prof(PROF_GEMM, st, flops);
-    if (d.a_kcontig && d.b_kcontig) k_gemm<true, true, BN_, STAGES_><<<grid, block, SMEM, st>>>(d);
-    else if (d.a_kcontig) k_gemm<true, false, BN_, STAGES_><<<grid, block, SMEM, st>>>(d);
-    else if (d.b_kcontig) k_gemm<false, true, BN_, STAGES_><<<grid, block, SMEM, st>>>(d);
-    else k_gemm<false, false, BN_, STAGES_><<<grid, block, SMEM, st>>>(d);
+    ProfScope prof(PROF_GEMM, st, flops * d.nb);
+    if (d.nb > 1) {
+        if (d.a_kcontig && d.b_kcontig) k_gemm<true, true, BN_, STAGES_, true><<<grid, block, SMEM, st>>>(d);
+        else if (d.a_kcontig) k_gemm<true, false, BN_, STAGES_, true><<<grid, block, SMEM, st>>>(d);
+        else if (d.b_kcontig) k_gemm<false, true, BN_, STAGES_, true><<<grid, block, SMEM, st>>>(d);
+        else k_gemm<false, false, BN_, STAGES_, true><<<grid, block, SMEM, st>>>(d);
+    } else {
+        if (d.a_kcontig && d.b_kcontig) k_gemm<true, true, BN_, STAGES_, false><<<grid, block, SMEM, st>>>(d);
+        else if (d.a_kcontig) k_gemm<true, false, BN_, STAGES_, false><<<grid, block, SMEM, st>>>(d);
+        else if (d.b_kcontig) k_gemm<false, true, BN_, STAGES_, false><<<grid, block, SMEM, st>>>(d);
+        else k_gemm<false, false, BN_, STAGES_, false><<<grid, block, SMEM, st>>>(d);
+    }
     count_launch();
     return PIGP_OK;
 }
@@ -670,8 +702,9 @@ int launch_gemm(const GemmDesc& g_in, cudaStream_t st) {
         return PIGP_EINVAL;
     }
     if (g.m_ts == 0) g.m_ts = 1;
+    if (g.nb <= 0) g.nb = 1;
     if (g.Lkk) {
-        if (g.N != BM || g.K != BM || !g.a_kcontig || !g.b_kcontig || g.C != g.A || g.alpha != 1.0 || g.beta != 0.0) {
+        if (g.N != BM || g.K != BM || !g.a_kcontig || !g.b_kcontig || g.C != g.A || g.sc != g.sa || g.alpha != 1.0 || g.beta != 0.0) {
             set_error("pigp gemm: the block TRSM is in place with N = K = 128 and k-contiguous operands");
             return PIGP_EINVAL;
         }
@@ -929,8 +962,14 @@ __device__ __noinline__ void warp_inverse32(const double* D, int ld, double* Win
 // inv(L) (lower, zeros above) to invd[128*128].  Non-positive pivot -> *info = base + column + 1 (first one wins)
 // and NaNs propagate, which is what jnp.linalg.cholesky gives the reference.
 // Peers (multi-GPU) receive inv(L) and the diagonal of L -- what their TRSMs and their log-det read -- then the flag.
-__global__ void __launch_bounds__(256, 1) k_potf2(double* A, int64_t ld, double* invd, int32_t* info, int base) {
+template <bool BATCH>
+__global__ void __launch_bounds__(256, 1) k_potf2(double* A, int64_t ld, double* invd, int32_t* info, int base, int64_t sA, int64_t sI) {
     extern __shared__ __align__(16) double sm[];
+    if (BATCH) {
+        A += blockIdx.y * sA;
+        invd += blockIdx.y * sI;
+        if (info) info += blockIdx.y;
+    }
     double* scratch = sm + PT * PLD;
     double* xch = scratch + N_SCRATCH * 32 * SLD;    // exchange area of warp_factor32: 2 x 32 x 4 doubles
     double* rdiag = xch + 2 * 32 * 4;                 // 1 / L_ii of the block being factored
@@ -1031,8 +1070,15 @@ __global__ void __launch_bounds__(256, 1) k_potf2(double* A, int64_t ld, double*
 //   the two 64 x 64 diagonal halves from their 32-blocks, W_ba = -inv(L_b) (L_ba inv(L_a)); then W21 = -W22 (L21 W11), with
 //   the (unused) upper-right 64 x 64 quadrant of the tile as scratch for L21 W11.
 // Optionally also writes the tile transposed into Yt (the diagonal tile of Y = L^-T, zeros below its diagonal).
-__global__ void __launch_bounds__(256, 1) k_tile_inv(const double* L, int64_t ld, double* invd, int first, int stride, double* Y, int64_t ldy, int zero_upper) {
+template <bool BATCH>
+__global__ void __launch_bounds__(256, 1) k_tile_inv(const double* L, int64_t ld, double* invd, int first, int stride, double* Y, int64_t ldy,
+                                                      int zero_upper, int64_t sL, int64_t sI, int64_t sY) {
     extern __shared__ __align__(16) double sm[];
+    if (BATCH) {
+        L += blockIdx.y * sL;
+        invd += blockIdx.y * sI;
+        if (Y) Y += blockIdx.y * sY;
+    }
     double* scratch = sm + PT * PLD;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int c = first + blockIdx.x * stride;
@@ -1112,17 +1158,21 @@ __global__ void __launch_bounds__(256, 1) k_tile_inv(const double* L, int64_t ld
     }
 }
 
-int launch_tile_inv(const double* L, int64_t ld, double* invd, int first, int stride, int count, double* Y, int64_t ldy, cudaStream_t st, int zero_upper) {
+int launch_tile_inv(const double* L, int64_t ld, double* invd, int first, int stride, int count, double* Y, int64_t ldy, cudaStream_t st, int zero_upper,
+                    int nb, int64_t sL, int64_t sI, int64_t sY) {
     if (count <= 0) return PIGP_OK;
     static bool attr_done[64] = {};
     int dev = 0;
     PIGP_CUDA(cudaGetDevice(&dev));
     if (!attr_done[dev & 63]) {
-        PIGP_CUDA(cudaFuncSetAttribute(k_tile_inv, cudaFuncAttributeMaxDynamicSharedMemorySize, POTF2_SMEM));
+        PIGP_CUDA(cudaFuncSetAttribute(k_tile_inv<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, POTF2_SMEM));
+        PIGP_CUDA(cudaFuncSetAttribute(k_tile_inv<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, POTF2_SMEM));
         attr_done[dev & 63] = true;
     }
     ProfScope prof(PROF_POTF2, st);
-    k_tile_inv<<<(unsigned)count, 256, POTF2_SMEM, st>>>(L, ld, invd, first, stride, Y, ldy, zero_upper);
+    const dim3 grid((unsigned)count, (unsigned)nb);
+    if (nb > 1) k_tile_inv<true><<<grid, 256, POTF2_SMEM, st>>>(L, ld, invd, first, stride, Y, ldy, zero_upper, sL, sI, sY);
+    else k_tile_inv<false><<<grid, 256, POTF2_SMEM, st>>>(L, ld, invd, first, stride, Y, ldy, zero_upper, sL, sI, sY);
     count_launch();
     PIGP_CUDA(cudaGetLastError());
     return PIGP_OK;
@@ -1133,17 +1183,19 @@ int set_potf2_debug(long long* dev_buf) {
     return PIGP_OK;
 }
 
-int launch_potf2(double* A, int64_t ld, double* invd, int32_t* info, int base, cudaStream_t st) {
+int launch_potf2(double* A, int64_t ld, double* invd, int32_t* info, int base, cudaStream_t st, int nb, int64_t sA, int64_t sI) {
     static bool attr_done[64] = {};
     int dev = 0;
     PIGP_CUDA(cudaGetDevice(&dev));
     bool& attr_set = attr_done[dev & 63];
     if (!attr_set) {
-        PIGP_CUDA(cudaFuncSetAttribute(k_potf2, cudaFuncAttributeMaxDynamicSharedMemorySize, POTF2_SMEM));
+        PIGP_CUDA(cudaFuncSetAttribute(k_potf2<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, POTF2_SMEM));
+        PIGP_CUDA(cudaFuncSetAttribute(k_potf2<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, POTF2_SMEM));
         attr_set = true;
     }
     ProfScope prof(PROF_POTF2, st);
-    k_potf2<<<1, 256, POTF2_SMEM, st>>>(A, ld, invd, info, base);
+    if (nb > 1) k_potf2<true><<<dim3(1, (unsigned)nb), 256, POTF2_SMEM, st>>>(A, ld, invd, info, base, sA, sI);
+    else k_potf2<false><<<1, 256, POTF2_SMEM, st>>>(A, ld, invd, info, base, sA, sI);
     count_launch();
     PIGP_CUDA(cudaGetLastError());
     return PIGP_OK;
@@ -1214,8 +1266,12 @@ int potri_lower(const double* L, int64_t ld, int64_t n, const double* invd, doub
 
 // ----------------------------------------------------------------------------------------------- reductions / BLAS-2
 // out2[0] = sum_{i<n} log A[i][i],  out2[1] = sum_{j<n} v[j]^2   (single CTA, fixed order: deterministic)
-__global__ void __launch_bounds__(1024) k_logdet_quad(const double* A, int64_t ld, int64_t n, const double* v, double* out2) {
+__global__ void __launch_bounds__(1024) k_logdet_quad(const double* A, int64_t ld, int64_t n, const double* v, double* out2, int64_t sA,
+                                                      int64_t sv) {
     __shared__ double sh[2][32];
+    A += blockIdx.y * sA;
+    v += blockIdx.y * sv;
+    out2 += 2 * blockIdx.y;
     double s0 = 0.0, s1 = 0.0;
     for (int64_t i = threadIdx.x; i < n; i += blockDim.x) {
         s0 += log(A[i * ld + i]);
@@ -1241,9 +1297,10 @@ __global__ void __launch_bounds__(1024) k_logdet_quad(const double* A, int64_t l
     }
 }
 
-int launch_logdet_quad(const double* A, int64_t ld, int64_t n, const double* v, double* out2, cudaStream_t st) {
+int launch_logdet_quad(const double* A, int64_t ld, int64_t n, const double* v, double* out2, cudaStream_t st, int nb, int64_t sA,
+                       int64_t sv) {
     ProfScope prof(PROF_MISC, st);
-    k_logdet_quad<<<1, 1024, 0, st>>>(A, ld, n, v, out2);
+    k_logdet_quad<<<dim3(1, (unsigned)nb), 1024, 0, st>>>(A, ld, n, v, out2, sA, sv);
     count_launch();
     PIGP_CUDA(cudaGetLastError());
     return PIGP_OK;
@@ -1280,24 +1337,26 @@ int launch_gemv(const double* A, int64_t ld, int64_t m, int64_t n, const double*
 }
 
 int preload_dense() {
-    PIGP_CUDA(cudaFuncSetAttribute(k_gemm_s<32, 128, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, 3 * (32 + 128) * LDS_K * (int)sizeof(double)));
-    PIGP_CUDA(cudaFuncSetAttribute(k_gemm_s<64, 64, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, 3 * (64 + 64) * LDS_K * (int)sizeof(double)));
-    PIGP_CUDA(cudaFuncSetAttribute(k_gemm_s<32, 64, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, 3 * (32 + 64) * LDS_K * (int)sizeof(double)));
-    PIGP_PRELOAD((k_gemm_s<32, 128, 3>));
-    PIGP_PRELOAD((k_gemm_s<64, 64, 3>));
-    PIGP_PRELOAD((k_gemm_s<32, 64, 3>));
-    PIGP_CUDA(cudaFuncSetAttribute(k_trsm_blk<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, tb_smem(8)));
-    PIGP_CUDA(cudaFuncSetAttribute(k_trsm_blk<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, tb_smem(16)));
-    PIGP_CUDA(cudaFuncSetAttribute(k_trsm_blk<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, tb_smem(32)));
-    PIGP_PRELOAD(k_trsm_blk<8>);
-    PIGP_PRELOAD(k_trsm_blk<16>);
-    PIGP_PRELOAD(k_trsm_blk<32>);
+    // (the batched instantiations of k_gemm_s / k_trsm_blk / k_potf2 / k_tile_inv are left to their launchers: a batch never
+    // runs on a multi-rank solver, whose creation is what this is for)
+    PIGP_CUDA(cudaFuncSetAttribute(k_gemm_s<32, 128, 3, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 3 * (32 + 128) * LDS_K * (int)sizeof(double)));
+    PIGP_CUDA(cudaFuncSetAttribute(k_gemm_s<64, 64, 3, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 3 * (64 + 64) * LDS_K * (int)sizeof(double)));
+    PIGP_CUDA(cudaFuncSetAttribute(k_gemm_s<32, 64, 3, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 3 * (32 + 64) * LDS_K * (int)sizeof(double)));
+    PIGP_PRELOAD((k_gemm_s<32, 128, 3, false>));
+    PIGP_PRELOAD((k_gemm_s<64, 64, 3, false>));
+    PIGP_PRELOAD((k_gemm_s<32, 64, 3, false>));
+    PIGP_CUDA(cudaFuncSetAttribute(k_trsm_blk<8, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, tb_smem(8)));
+    PIGP_CUDA(cudaFuncSetAttribute(k_trsm_blk<16, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, tb_smem(16)));
+    PIGP_CUDA(cudaFuncSetAttribute(k_trsm_blk<32, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, tb_smem(32)));
+    PIGP_PRELOAD((k_trsm_blk<8, false>));
+    PIGP_PRELOAD((k_trsm_blk<16, false>));
+    PIGP_PRELOAD((k_trsm_blk<32, false>));
     PIGP_TRY((gemm_attrs<128, 4>()));
     PIGP_TRY((gemm_attrs<64, 3>()));
-    PIGP_CUDA(cudaFuncSetAttribute(k_potf2, cudaFuncAttributeMaxDynamicSharedMemorySize, POTF2_SMEM));
-    PIGP_PRELOAD(k_potf2);
-    PIGP_CUDA(cudaFuncSetAttribute(k_tile_inv, cudaFuncAttributeMaxDynamicSharedMemorySize, POTF2_SMEM));
-    PIGP_PRELOAD(k_tile_inv);
+    PIGP_CUDA(cudaFuncSetAttribute(k_potf2<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, POTF2_SMEM));
+    PIGP_PRELOAD(k_potf2<false>);
+    PIGP_CUDA(cudaFuncSetAttribute(k_tile_inv<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, POTF2_SMEM));
+    PIGP_PRELOAD(k_tile_inv<false>);
     PIGP_PRELOAD(k_place_diag);
     PIGP_PRELOAD(k_logdet_quad);
     PIGP_PRELOAD(k_gemv);

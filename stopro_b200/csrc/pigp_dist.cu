@@ -117,8 +117,13 @@ __global__ void __launch_bounds__(256) k_push_diag(const double* invk, const dou
     push_done(sg);
 }
 
+// The small kernels below take one grid dimension (y) more per batch slot b: b's vectors of npad entries follow each other,
+// its matrices are at + b * sL (L and its y tile) or + b * sY (Y).
 // alpha[j] = sum_{k >= tile(j) * 128} Y[j][k] v[k]   (one warp per row; Y upper triangular by tiles)
-__global__ void __launch_bounds__(256) k_gemv_upper(const double* Y, int64_t ld, int64_t npad, const double* v, double* alpha) {
+__global__ void __launch_bounds__(256) k_gemv_upper(const double* Y, int64_t ld, int64_t npad, const double* v, double* alpha, int64_t sY) {
+    Y += blockIdx.y * sY;
+    v += blockIdx.y * npad;
+    alpha += blockIdx.y * npad;
     const int64_t row = (int64_t)blockIdx.x * 8 + (threadIdx.x >> 5);
     if (row >= npad) return;
     const int lane = threadIdx.x & 31;
@@ -139,7 +144,8 @@ __global__ void __launch_bounds__(256) k_gemv_upper(const double* Y, int64_t ld,
 }
 
 // own y tile: first row = [y, 0 ...], other rows zero
-__global__ void __launch_bounds__(256) k_set_ytile(double* tile, int64_t ld, int64_t n, int64_t npad, const double* y) {
+__global__ void __launch_bounds__(256) k_set_ytile(double* tile, int64_t ld, int64_t n, int64_t npad, const double* y, int64_t sL) {
+    tile += blockIdx.y * sL;
     const int64_t total = 128 * npad;
     for (int64_t e = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; e < total; e += (int64_t)gridDim.x * blockDim.x) {
         const int64_t r = e / npad, c = e % npad;
@@ -147,17 +153,22 @@ __global__ void __launch_bounds__(256) k_set_ytile(double* tile, int64_t ld, int
     }
 }
 
-__global__ void k_push_vec(const double* src, int len, int slot, double* local_slots, PeerBufs pb) {
+__global__ void k_push_vec(const double* src, int len, int slot, double* local_slots, PeerBufs pb, int64_t s_slots) {
     const int i = threadIdx.x;
     if (i >= len) return;
+    src += blockIdx.y * MAX_THETA;
+    local_slots += blockIdx.y * s_slots;
     const double v = src[i];
     local_slots[slot * MAX_THETA + i] = v;
     for (int p = 0; p < pb.n; ++p) pb.p[p][slot * MAX_THETA + i] = v;
 }
 
-__global__ void k_sum_slots(const double* slots, int world, int len, double* out, const int32_t* info, const int* err) {
+__global__ void k_sum_slots(const double* slots, int world, int len, double* out, const int32_t* info, const int* err, int64_t s_slots) {
     const int i = threadIdx.x;
     if (i >= len) return;
+    slots += blockIdx.y * s_slots;
+    out += blockIdx.y * len;
+    if (info) info += blockIdx.y;
     double s = 0.0;
     for (int r = 0; r < world; ++r) s += slots[r * MAX_THETA + i];  // rank order: same result on every rank
     if ((info && *info != 0) || (err && *err != 0)) s = nan("");
@@ -165,6 +176,9 @@ __global__ void k_sum_slots(const double* slots, int world, int len, double* out
 }
 
 __global__ void k_finish_nll_d(const double* out2, int64_t n, int32_t* info, const int* err, double* nll) {
+    out2 += 2 * blockIdx.y;
+    info += blockIdx.y;
+    nll += blockIdx.y;
     double v = 0.5 * out2[1] + out2[0] + 0.5 * (double)n * log(2.0 * 3.14159265358979323846);  // GP/gp.py:85-89
     if (err && *err != 0) *info = -1;  // a peer's flag never arrived: reported through info (device-pointer API) as well
     if (*info != 0) v = nan("");
@@ -173,8 +187,10 @@ __global__ void k_finish_nll_d(const double* out2, int64_t n, int32_t* info, con
 
 // info <- 1-based index of the first diagonal entry of the replicated factor that is not a positive number (0: none).
 // Every rank derives the same value from its copy of L (the owner's k_potf2 saw the pivot itself).
-__global__ void __launch_bounds__(1024) k_diag_info(const double* L, int64_t ld, int64_t n, int32_t* info) {
+__global__ void __launch_bounds__(1024) k_diag_info(const double* L, int64_t ld, int64_t n, int32_t* info, int64_t sL) {
     __shared__ int best;
+    L += blockIdx.y * sL;
+    info += blockIdx.y;
     if (threadIdx.x == 0) best = 0x7fffffff;
     __syncthreads();
     int mine = 0x7fffffff;
@@ -185,7 +201,9 @@ __global__ void __launch_bounds__(1024) k_diag_info(const double* L, int64_t ld,
     if (threadIdx.x == 0) *info = (best == 0x7fffffff) ? 0 : best;
 }
 
-__global__ void k_copy_v(const double* row, int64_t npad, double* v) {
+__global__ void k_copy_v(const double* row, int64_t npad, double* v, int64_t sL) {
+    row += blockIdx.y * sL;
+    v += blockIdx.y * npad;
     const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (i < npad) v[i] = row[i];
 }
@@ -301,6 +319,11 @@ struct pigp_dsolver {
     int k_done = 0;
     cudaStream_t se = nullptr;  // completes the inverse diagonal tiles (k_tile_inv) as soon as L_kk exists, off both chains
     PanelSched panels{true};
+    // batch workspace (world = 1; Work below): per-slot copies of L with its y tile, invd and the small vectors, grown to the
+    // largest batch seen; Y and K^-1 separately, to the largest batch that needed them
+    int b_cap = 0, b_cap_y = 0, b_cap_k = 0;
+    double *bL = nullptr, *binvd = nullptr, *bvec = nullptr, *bY = nullptr, *bK = nullptr;
+    int32_t* binfo = nullptr;
 
     int f_diag(int k) const { return k; }
     int f_panel(int k, int src) const { return T + k * world + src; }
@@ -317,15 +340,31 @@ FactorView factor_view(pigp_dsolver* s) {
     f.end = s->gy + 1;  // this rank's y tile rides through the TRSMs: L^-1 y comes out of the same launches
     f.rank = s->rank; f.world = s->world;
     f.v = s->L + (int64_t)s->gy * TILE * s->ld;  // first row of the y tile: L^-1 y after the factorisation
+    f.nb = 1; f.sL = (int64_t)(s->T + s->world) * TILE * s->ld; f.sI = (int64_t)s->T * TILE * TILE;
     return f;
 }
 }  // namespace pigp
 
 namespace {
 
+// The buffers one evaluation works in.  A single-theta call uses the solver's own (nb = 1); a batch of nb slots uses the
+// batch workspace, where slot b's copy of a buffer is at + b * its stride: sL for L, sI for invd, sY for Y and K^-1,
+// npad for v and alpha, 2 for out2, one per slot for info, max(n_tiles, 1) * MAX_THETA for partials, MAX_THETA for gpart
+// and world * MAX_THETA for gslots.
+struct Work {
+    int nb;
+    double* L; int64_t sL;      // (T + world) * 128 rows x ld: K -> L, the y tile below it
+    double* invd; int64_t sI;
+    double *Y, *Kinv; int64_t sY;  // npad x ld each; only with the gradient (K^-1 only with the early products)
+    double *partials, *gpart, *gslots, *out2, *v, *alpha;
+    int32_t* info;
+};
+
 struct Ctx {
     FactorView f;      // the matrix being factored
     pigp_dsolver* s;   // everything else of the solver: only with grad or peers (null under pigp_potrf_lower)
+    double *Y, *Kinv;  // L^-T and the early K^-1 (grad only); slot b at + b * sY
+    int64_t sY;
     cudaStream_t st;   // chain stream
     cudaStream_t sb;   // side stream (Y = L^-T), used when grad is set
     cudaStream_t sc;   // publication stream
@@ -339,9 +378,12 @@ struct Ctx {
     int others[7];
 };
 
-Ctx make_ctx(pigp_dsolver* s, cudaStream_t st) {
+Ctx make_ctx(pigp_dsolver* s, cudaStream_t st, const Work& w) {
     Ctx c{};
     c.f = factor_view(s); c.s = s; c.st = st;
+    c.f.L = w.L; c.f.invd = w.invd; c.f.info = w.info; c.f.v = w.L + (int64_t)s->gy * TILE * s->ld;
+    c.f.nb = w.nb; c.f.sL = w.sL; c.f.sI = w.sI;
+    c.Y = w.Y; c.Kinv = w.Kinv; c.sY = w.sY;
     int k = 0;
     for (int p = 0; p < s->world; ++p)
         if (p != s->rank) { c.others[k] = p; c.pf.f[k] = s->peer(p, s->flags); ++k; }
@@ -404,6 +446,11 @@ PushSig make_sig(const Ctx& c, int idx) {
     return sg;
 }
 
+// every slot of a batch runs the same product: A, B, C (and Lkk) in buffers of these per-slot strides
+void set_slots(GemmDesc& g, const Ctx& c, int64_t sa, int64_t sb, int64_t sc, int64_t sl = 0) {
+    g.nb = c.f.nb; g.sa = sa; g.sb = sb; g.sc = sc; g.sl = sl;
+}
+
 int leaf(const Ctx& c, int k) {
     const FactorView& f = c.f;
     pigp_dsolver* s = c.s;
@@ -411,7 +458,7 @@ int leaf(const Ctx& c, int k) {
     double* invk = f.invd + (int64_t)k * TILE * TILE;
     double* Akk = f.L + (int64_t)k * TILE * ld + (int64_t)k * TILE;
     const bool mine = (k % f.world == f.rank), multi = c.npeers > 0;
-    if (mine) PIGP_TRY(launch_potf2(Akk, ld, invk, f.info, k * TILE, c.st));
+    if (mine) PIGP_TRY(launch_potf2(Akk, ld, invk, f.info, k * TILE, c.st, f.nb, f.sL, f.sI));
     if (c.grad || multi) PIGP_CUDA(cudaEventRecord(s->ev_diag[k], c.st));  // mine: inv(L_kk) is ready; else: the chain has reached leaf k
     if (mine && multi) {
         // publish inv(L_kk) and diag(L_kk) from the publication stream while the chain goes on with this rank's own TRSM
@@ -438,6 +485,7 @@ int leaf(const Ctx& c, int k) {
             g.gen = 1; g.m_ts = f.world; g.m_gt0 = first; g.n_gt0 = k; g.k_gt0 = k;
             g.force_bn128 = 1;  // in place
             g.Lkk = Akk; g.ldl = ld;  // refined: needs L_kk itself next to its inverse (peers receive both)
+            set_slots(g, c, f.sL, f.sI, f.sL, f.sL);
             if (!mine) PIGP_TRY(set_wait_one(c, g, s->f_diag(k), c.st));
             PIGP_TRY(launch_gemm(g, c.st));
         }
@@ -465,7 +513,7 @@ int leaf(const Ctx& c, int k) {
         // (on its own stream: it depends on L_kk only, so it runs ahead of the L^-T chain instead of inside it)
         PIGP_CUDA(cudaStreamWaitEvent(c.se, s->ev_diag[k], 0));
         if (!mine) PIGP_TRY(wait_one(c, s->f_diag(k), c.se));
-        PIGP_TRY(launch_tile_inv(s->L, ld, s->invd, k, 1, 1, mine ? s->Y : nullptr, ld, c.se));
+        PIGP_TRY(launch_tile_inv(f.L, ld, f.invd, k, 1, 1, mine ? c.Y : nullptr, ld, c.se, 0, f.nb, f.sL, f.sI, c.sY));
         PIGP_CUDA(cudaEventRecord(s->ev_inv[k], c.se));
         PIGP_CUDA(cudaStreamWaitEvent(c.sb, s->ev_inv[k], 0));
         const int first = f.first_own(0), cnt = f.count_own(0, k);
@@ -473,12 +521,13 @@ int leaf(const Ctx& c, int k) {
             GemmDesc g{};
             g.M = cnt * TILE; g.N = TILE; g.K = TILE;
             g.alpha = 1.0; g.beta = 0.0;
-            double* Cb = s->Y + (int64_t)first * TILE * ld + (int64_t)k * TILE;
+            double* Cb = c.Y + (int64_t)first * TILE * ld + (int64_t)k * TILE;
             g.A = Cb; g.lda = ld; g.a_kcontig = 1;
             g.B = invk; g.ldb = TILE; g.b_kcontig = 1;
             g.C = Cb; g.ldc = ld;
             g.gen = 1; g.m_ts = s->world; g.m_gt0 = first; g.n_gt0 = k; g.k_gt0 = k;
             g.force_bn128 = 1;
+            set_slots(g, c, c.sY, f.sI, c.sY);
             PIGP_TRY(launch_gemm(g, c.sb));
         }
         // columns [k_done, k + 1) of Y are final once the side stream gets here: their share of K^-1 = Y Y^T,
@@ -491,11 +540,12 @@ int leaf(const Ctx& c, int k) {
             GemmDesc g{};
             g.M = b * TILE; g.N = b * TILE; g.K = (b - a) * TILE;
             g.alpha = 1.0; g.beta = 1.0;
-            g.A = s->Y + (int64_t)a * TILE; g.lda = ld; g.a_kcontig = 1;
-            g.B = s->Y + (int64_t)a * TILE; g.ldb = ld; g.b_kcontig = 1;
-            g.C = s->Kinv; g.ldc = ld;
+            g.A = c.Y + (int64_t)a * TILE; g.lda = ld; g.a_kcontig = 1;
+            g.B = c.Y + (int64_t)a * TILE; g.ldb = ld; g.b_kcontig = 1;
+            g.C = c.Kinv; g.ldc = ld;
             g.lower_only = 1; g.kmode = 1;
             g.gen = 1; g.m_ts = 1; g.m_gt0 = 0; g.n_gt0 = 0; g.k_gt0 = a;
+            set_slots(g, c, c.sY, c.sY, c.sY);
             PIGP_TRY(launch_gemm(g, c.sk));
             s->k_done = b;
         }
@@ -523,6 +573,7 @@ int rec(const Ctx& c, int c0, int nt) {
             g.C = f.L + (int64_t)first * TILE * ld + (int64_t)(c0 + n1) * TILE; g.ldc = ld;
             g.lower_only = 1;
             g.gen = 1; g.m_ts = f.world; g.m_gt0 = first; g.n_gt0 = c0 + n1; g.k_gt0 = c0;
+            set_slots(g, c, f.sL, f.sL, f.sL);
             if (c.npeers > 0) PIGP_TRY(set_wait_all(c, g, s->f_panel(k1, 0), c.st));
             PIGP_TRY(launch_gemm(g, c.st));
         }
@@ -535,11 +586,12 @@ int rec(const Ctx& c, int c0, int nt) {
             GemmDesc g{};
             g.M = cnt * TILE; g.N = n2 * TILE; g.K = n1 * TILE;
             g.alpha = -1.0; g.beta = 1.0;
-            g.A = s->Y + (int64_t)first * TILE * ld + (int64_t)c0 * TILE; g.lda = ld; g.a_kcontig = 1;
-            g.B = s->L + (int64_t)(c0 + n1) * TILE * ld + (int64_t)c0 * TILE; g.ldb = ld; g.b_kcontig = 1;
-            g.C = s->Y + (int64_t)first * TILE * ld + (int64_t)(c0 + n1) * TILE; g.ldc = ld;
+            g.A = c.Y + (int64_t)first * TILE * ld + (int64_t)c0 * TILE; g.lda = ld; g.a_kcontig = 1;
+            g.B = f.L + (int64_t)(c0 + n1) * TILE * ld + (int64_t)c0 * TILE; g.ldb = ld; g.b_kcontig = 1;
+            g.C = c.Y + (int64_t)first * TILE * ld + (int64_t)(c0 + n1) * TILE; g.ldc = ld;
             g.kmode = 1;
             g.gen = 1; g.m_ts = s->world; g.m_gt0 = first; g.n_gt0 = c0 + n1; g.k_gt0 = c0;
+            set_slots(g, c, c.sY, f.sL, c.sY);
             PIGP_TRY(set_wait_all(c, g, s->f_panel(k1, 0), c.sb));
             // Optionally issued in k-chunks (PIGP_SIDE_CHUNK = tiles per launch): a CTA of a K = 10k product holds its SM
             // slot for ~1 ms, and the chain's (and the publication stream's) small high-priority kernels can only start
@@ -596,6 +648,7 @@ static int panel_update(const Ctx& c, int k0, int k1, int jc0, int jc1, cudaStre
     g.C = f.L + (int64_t)first * TILE * ld + (int64_t)jc0 * TILE; g.ldc = ld;
     g.lower_only = 1;
     g.gen = 1; g.m_ts = f.world; g.m_gt0 = first; g.n_gt0 = jc0; g.k_gt0 = k0;
+    set_slots(g, c, f.sL, f.sL, f.sL);
     return launch_gemm(g, st);
 }
 
@@ -627,11 +680,12 @@ static int chol_lookahead(const Ctx& c, int W, PanelSched& ps) {
                 GemmDesc g{};
                 g.M = cnt * TILE; g.N = (T - j1) * TILE; g.K = (j1 - j0) * TILE;
                 g.alpha = -1.0; g.beta = 1.0;
-                g.A = s->Y + (int64_t)first * TILE * ld + (int64_t)j0 * TILE; g.lda = ld; g.a_kcontig = 1;
-                g.B = s->L + (int64_t)j1 * TILE * ld + (int64_t)j0 * TILE; g.ldb = ld; g.b_kcontig = 1;
-                g.C = s->Y + (int64_t)first * TILE * ld + (int64_t)j1 * TILE; g.ldc = ld;
+                g.A = c.Y + (int64_t)first * TILE * ld + (int64_t)j0 * TILE; g.lda = ld; g.a_kcontig = 1;
+                g.B = f.L + (int64_t)j1 * TILE * ld + (int64_t)j0 * TILE; g.ldb = ld; g.b_kcontig = 1;
+                g.C = c.Y + (int64_t)first * TILE * ld + (int64_t)j1 * TILE; g.ldc = ld;
                 g.kmode = 1;
                 g.gen = 1; g.m_ts = s->world; g.m_gt0 = first; g.n_gt0 = j1; g.k_gt0 = j0;
+                set_slots(g, c, c.sY, f.sL, c.sY);
                 PIGP_TRY(launch_gemm(g, c.sb));
             }
         }
@@ -669,6 +723,7 @@ int pigp::potrf_lower(double* A, int64_t ld, int64_t n, int64_t m_extra, double*
     c.f.L = A; c.f.ld = ld; c.f.invd = invd; c.f.info = info;
     c.f.T = (int)(n / TILE); c.f.end = (int)((n + m_extra) / TILE);
     c.f.rank = 0; c.f.world = 1;
+    c.f.nb = 1;
     const int W = lookahead_width(c.f.T, 1, false);
     if (W > 0 && c.f.T > W) {
         int dev = 0;
@@ -704,6 +759,7 @@ void pigp_dsolver_destroy(pigp_dsolver* s) {
     if (s->ev_k) cudaEventDestroy(s->ev_k);
     if (s->ev_kd) cudaEventDestroy(s->ev_kd);
     cudaFree(s->Kinv);
+    cudaFree(s->bL); cudaFree(s->binvd); cudaFree(s->bvec); cudaFree(s->bY); cudaFree(s->bK); cudaFree(s->binfo);
     delete s;
 }
 
@@ -878,12 +934,96 @@ int pigp_device_uuid(void* out16) {
     return PIGP_OK;
 }
 
-static int dsolver_enqueue(pigp_dsolver* s, const double* theta_dev, const double* y_dev, double eps, double* nll_dev,
-                           double* grad_dev, int32_t* info_dev, cudaStream_t st);
+// PIGP_EARLY_KINV=0 switches the early K^-1 products off.  Worth it while the evaluation is latency bound and its GEMMs
+// are short: -9 % at N = 1180, -7.5 % at 2640.  From N ~ 5000 on nothing is gained (measured 5018 ... 12700): the
+// product's CTAs then hold every SM for tens of microseconds, and each of the chains' launches waits that long for a slot
+// -- priorities do not pre-empt
+static bool early_kinv_on(const pigp_dsolver* s, bool grad) {
+    static int early = -1;
+    if (early < 0) { const char* e = getenv("PIGP_EARLY_KINV"); early = (e && atoi(e) == 0) ? 0 : 1; }
+    return early && grad && s->world == 1 && s->T >= 8 && s->T <= 32;
+}
 
-int pigp_dsolver_nll_grad(pigp_dsolver* s, const double* theta_dev, const double* y_dev, double eps, double* nll_dev,
-                          double* grad_dev, int32_t* info_dev, void* stream) {
-    if (!s || !theta_dev || !y_dev || !nll_dev) { set_error("pigp_dsolver_nll_grad: null argument"); return PIGP_EINVAL; }
+// the solver's own buffers (one slot); Y (world = 1) and K^-1 are allocated on the first call that needs them
+static int own_work(pigp_dsolver* s, bool grad, Work& w) {
+    if (grad && !s->Y) PIGP_CUDA(cudaMalloc(&s->Y, sizeof(double) * (size_t)s->npad * s->ld));
+    if (early_kinv_on(s, grad) && !s->Kinv) PIGP_CUDA(cudaMalloc(&s->Kinv, sizeof(double) * (size_t)s->npad * s->ld));
+    const FactorView f = factor_view(s);
+    w = Work{};
+    w.nb = 1;
+    w.L = s->L; w.sL = f.sL; w.invd = s->invd; w.sI = f.sI;
+    w.Y = s->Y; w.Kinv = s->Kinv; w.sY = s->npad * s->ld;
+    w.partials = s->partials; w.gpart = s->gpart; w.gslots = s->gslots; w.out2 = s->out2; w.v = s->v; w.alpha = s->alpha;
+    w.info = s->info;
+    return PIGP_OK;
+}
+
+// per-slot vectors of the batch workspace, one array each: partials, gpart, gslots, out2, v, alpha
+static int64_t vec_len(const pigp_dsolver* s) { return std::max<int64_t>(s->n_tiles, 1) * MAX_THETA + 2 * MAX_THETA + 2 + 2 * s->npad; }
+
+// Grow the batch workspace to nb slots.  Runs before anything is enqueued: on PIGP_ENOMEM nothing was launched, and the
+// solver stays usable for single calls and for the batches that still fit.  New buffers are zeroed on the caller's stream
+// `user`, which the schedule then waits for (the solver's own streams do not order with the legacy stream).
+static int batch_work(pigp_dsolver* s, int nb, bool grad, cudaStream_t user, Work& w) {
+    const FactorView f = factor_view(s);
+    const size_t mat = sizeof(double) * (size_t)s->npad * s->ld;
+    auto alloc = [&](void** p, size_t bytes) {
+        if (cudaMalloc(p, bytes) == cudaSuccess && cudaMemsetAsync(*p, 0, bytes, user) == cudaSuccess) return true;
+        cudaFree(*p);
+        *p = nullptr;
+        cudaGetLastError();  // not sticky: clear it, so that it is not reported by the next launch check
+        set_error("pigp_nll_grad_batch: out of device memory for the batch workspace");
+        return false;
+    };
+    if (nb > s->b_cap) {
+        cudaFree(s->bL); cudaFree(s->binvd); cudaFree(s->bvec); cudaFree(s->binfo);
+        s->bL = s->binvd = s->bvec = nullptr; s->binfo = nullptr;
+        s->b_cap = 0;
+        // zeroed once like the solver's slab: the parts of the inverse tiles above their diagonal blocks are read as zero
+        if (!alloc((void**)&s->bL, sizeof(double) * (size_t)f.sL * nb) || !alloc((void**)&s->binvd, sizeof(double) * (size_t)f.sI * nb) ||
+            !alloc((void**)&s->bvec, sizeof(double) * (size_t)vec_len(s) * nb) || !alloc((void**)&s->binfo, sizeof(int32_t) * (size_t)nb)) {
+            cudaFree(s->bL); cudaFree(s->binvd); cudaFree(s->bvec); cudaFree(s->binfo);
+            s->bL = s->binvd = s->bvec = nullptr; s->binfo = nullptr;
+            return PIGP_ENOMEM;
+        }
+        s->b_cap = nb;
+    }
+    if (grad && nb > s->b_cap_y) {
+        cudaFree(s->bY);
+        s->bY = nullptr;
+        s->b_cap_y = 0;
+        if (!alloc((void**)&s->bY, mat * nb)) return PIGP_ENOMEM;
+        s->b_cap_y = nb;
+    }
+    if (early_kinv_on(s, grad) && nb > s->b_cap_k) {
+        cudaFree(s->bK);
+        s->bK = nullptr;
+        s->b_cap_k = 0;
+        if (!alloc((void**)&s->bK, mat * nb)) return PIGP_ENOMEM;
+        s->b_cap_k = nb;
+    }
+    const int64_t cap = s->b_cap, pt = std::max<int64_t>(s->n_tiles, 1) * MAX_THETA;
+    w = Work{};
+    w.nb = nb;
+    w.L = s->bL; w.sL = f.sL; w.invd = s->binvd; w.sI = f.sI;
+    w.Y = s->bY; w.Kinv = s->bK; w.sY = s->npad * s->ld;
+    w.partials = s->bvec;
+    w.gpart = w.partials + cap * pt;
+    w.gslots = w.gpart + cap * MAX_THETA;
+    w.out2 = w.gslots + cap * MAX_THETA;
+    w.v = w.out2 + cap * 2;
+    w.alpha = w.v + cap * s->npad;
+    w.info = s->binfo;
+    return PIGP_OK;
+}
+
+static int dsolver_enqueue(pigp_dsolver* s, const Work& w, const double* theta_dev, const double* y_dev, double eps,
+                           double* nll_dev, double* grad_dev, int32_t* info_dev, cudaStream_t st);
+
+// One evaluation of w.nb slots: slot b reads theta_dev + b * theta_len and writes nll_dev + b, grad_dev + b * theta_len and
+// info_dev + b.  Every launch is issued once, for all slots.
+static int dsolver_call(pigp_dsolver* s, int nb, const double* theta_dev, const double* y_dev, double eps, double* nll_dev,
+                        double* grad_dev, int32_t* info_dev, void* stream) {
     if (!s->connected) { set_error("pigp_dsolver_nll_grad: peers are not connected"); return PIGP_EINVAL; }
     if (s->broken) { set_error("pigp_dsolver_nll_grad: an earlier call failed part-way; call pigp_dsolver_reset on every rank"); return PIGP_ECUDA; }
     cudaStream_t user = reinterpret_cast<cudaStream_t>(stream);
@@ -892,13 +1032,16 @@ int pigp_dsolver_nll_grad(pigp_dsolver* s, const double* theta_dev, const double
         int cur = -1;
         if (cudaGetDevice(&cur) == cudaSuccess && cur != s->plan->device) PIGP_CUDA(cudaSetDevice(s->plan->device));
     }
+    Work w;
+    if (nb == 1) PIGP_TRY(own_work(s, grad_dev != nullptr, w));
+    else PIGP_TRY(batch_work(s, nb, grad_dev != nullptr, user, w));
     PIGP_CUDA(cudaEventRecord(s->ev_in, user));
     PIGP_CUDA(cudaStreamWaitEvent(st, s->ev_in, 0));
     s->epoch += 1;
     // From here on the peers expect this rank's publications of epoch `epoch`: if an enqueue fails below, the call still
     // joins the user's stream to whatever was enqueued (so nothing runs unordered) and the solver is marked broken; the
     // peers' waits for the missing flags end at their time-out with info = -1 / NaN results.
-    const int rc = dsolver_enqueue(s, theta_dev, y_dev, eps, nll_dev, grad_dev, info_dev, st);
+    const int rc = dsolver_enqueue(s, w, theta_dev, y_dev, eps, nll_dev, grad_dev, info_dev, st);
     if (rc != PIGP_OK) s->broken = true;
     const cudaError_t e1 = cudaEventRecord(s->ev_out, st);
     const cudaError_t e2 = (e1 == cudaSuccess) ? cudaStreamWaitEvent(user, s->ev_out, 0) : e1;
@@ -907,11 +1050,30 @@ int pigp_dsolver_nll_grad(pigp_dsolver* s, const double* theta_dev, const double
     return PIGP_OK;
 }
 
-static int dsolver_enqueue(pigp_dsolver* s, const double* theta_dev, const double* y_dev, double eps, double* nll_dev,
-                           double* grad_dev, int32_t* info_dev, cudaStream_t st) {
+int pigp_dsolver_nll_grad(pigp_dsolver* s, const double* theta_dev, const double* y_dev, double eps, double* nll_dev,
+                          double* grad_dev, int32_t* info_dev, void* stream) {
+    if (!s || !theta_dev || !y_dev || !nll_dev) { set_error("pigp_dsolver_nll_grad: null argument"); return PIGP_EINVAL; }
+    return dsolver_call(s, 1, theta_dev, y_dev, eps, nll_dev, grad_dev, info_dev, stream);
+}
+
+}  // extern "C"
+
+int pigp::dsolver_nll_grad_batch(pigp_dsolver* s, int nb, const double* thetas_dev, const double* y_dev, double eps,
+                                 double* nll_dev, double* grad_dev, int32_t* info_dev, void* stream) {
+    if (!s || !thetas_dev || !y_dev || !nll_dev) { set_error("pigp_nll_grad_batch: null argument"); return PIGP_EINVAL; }
+    if (nb < 1 || nb > PIGP_MAX_BATCH) { set_error("pigp_nll_grad_batch: n_theta must be in [1, 65535]"); return PIGP_EINVAL; }
+    if (s->world != 1) { set_error("pigp_nll_grad_batch: sharded solvers (world > 1) evaluate one theta at a time"); return PIGP_EINVAL; }
+    return dsolver_call(s, nb, thetas_dev, y_dev, eps, nll_dev, grad_dev, info_dev, stream);
+}
+
+extern "C" {
+
+static int dsolver_enqueue(pigp_dsolver* s, const Work& w, const double* theta_dev, const double* y_dev, double eps,
+                           double* nll_dev, double* grad_dev, int32_t* info_dev, cudaStream_t st) {
     const pigp_plan* p = s->plan;
     const int64_t ld = s->ld;
-    Ctx c = make_ctx(s, st);
+    const int nb = w.nb, P = p->theta_len;
+    Ctx c = make_ctx(s, st, w);
     // serial mode: everything on the chain stream -- for the per-kernel timing pass, and for three or more ranks that share
     // one device (tests): the emulation would otherwise keep more streams with spinning waits alive than the device has
     // independent hardware queues, and a producer queued behind another rank's wait would dead-lock until the time-out
@@ -923,46 +1085,38 @@ static int dsolver_enqueue(pigp_dsolver* s, const double* theta_dev, const doubl
     c.se = serial ? st : (s->shared_device ? c.sb : s->se);
     c.grad = grad_dev != nullptr;
     c.sk = serial ? st : s->sk;
-    {
-        static int early = -1;  // PIGP_EARLY_KINV=0 switches the early products off
-        if (early < 0) { const char* e = getenv("PIGP_EARLY_KINV"); early = (e && atoi(e) == 0) ? 0 : 1; }
-        // worth it while the evaluation is latency bound and its GEMMs are short: -9 % at N = 1180, -7.5 % at 2640.  From
-        // N ~ 5000 on nothing is gained (measured 5018 ... 12700): the product's CTAs then hold every SM for tens of
-        // microseconds, and each of the chains' launches waits that long for a slot -- priorities do not pre-empt
-        c.early_kinv = early && c.grad && s->world == 1 && s->T >= 8 && s->T <= 32;
-        c.kinv_gran = std::max(2, s->T / 8);
-    }
-    int32_t* info = s->info;
-    PIGP_CUDA(cudaMemsetAsync(info, 0, sizeof(int32_t), st));
+    c.early_kinv = early_kinv_on(s, c.grad);
+    c.kinv_gran = std::max(2, s->T / 8);
+    int32_t* info = w.info;
+    PIGP_CUDA(cudaMemsetAsync(info, 0, sizeof(int32_t) * nb, st));
     // every peer has finished reading what the previous call left in this rank's buffers
     PIGP_TRY(signal(c, s->f_bar(s->rank)));
     PIGP_TRY(wait_all(c, s->f_bar(0), st, barrier_timeout_ns()));
     const int first = c.f.first_own(0), cnt = c.f.count_own(0, s->T);
-    if (c.grad && !s->Y) PIGP_CUDA(cudaMalloc(&s->Y, sizeof(double) * (size_t)s->npad * s->ld));
     if (c.grad) {
         PIGP_CUDA(cudaEventRecord(s->ev_bar, st));
         PIGP_CUDA(cudaStreamWaitEvent(c.sb, s->ev_bar, 0));
+        // (a batch has world = 1: its slots' Y follow each other, so their row tiles are one run of cnt * nb tiles)
         if (cnt > 0)
-            PIGP_CUDA(cudaMemset2DAsync(s->Y + (int64_t)first * TILE * ld, sizeof(double) * TILE * ld * s->world, 0,
-                                        sizeof(double) * TILE * ld, cnt, c.sb));
+            PIGP_CUDA(cudaMemset2DAsync(c.Y + (int64_t)first * TILE * ld, sizeof(double) * TILE * ld * s->world, 0,
+                                        sizeof(double) * TILE * ld, (size_t)cnt * nb, c.sb));
         // the inverse-tile stream writes the diagonal tiles of Y: behind the clearing of Y
         PIGP_CUDA(cudaEventRecord(s->ev_y0, c.sb));
         PIGP_CUDA(cudaStreamWaitEvent(c.se, s->ev_y0, 0));
         if (c.early_kinv) {
-            if (!s->Kinv) PIGP_CUDA(cudaMalloc(&s->Kinv, sizeof(double) * (size_t)s->npad * s->ld));
             PIGP_CUDA(cudaStreamWaitEvent(c.sk, s->ev_bar, 0));  // the previous evaluation's gradient kernel has read Kinv
-            PIGP_CUDA(cudaMemsetAsync(s->Kinv, 0, sizeof(double) * (size_t)s->npad * s->ld, c.sk));
+            PIGP_CUDA(cudaMemsetAsync(c.Kinv, 0, sizeof(double) * (size_t)s->npad * s->ld * nb, c.sk));
             s->k_done = 0;
         }
     }
     // own rows of K (lower, jitter added), identity padding (owner of the last tile), own y tile
-    PIGP_TRY(launch_assemble(p, s->d_tiles, s->n_tiles, theta_dev, eps, 1, s->L, ld, st));
+    PIGP_TRY(launch_assemble(p, s->d_tiles, s->n_tiles, theta_dev, eps, 1, w.L, ld, st, nb, P, w.sL));
     if (s->n < s->npad && (s->T - 1) % s->world == s->rank)
-        PIGP_TRY(launch_pad(s->L, ld, s->n, s->n, s->npad, s->npad, 1, 1, st));
-    double* ytile = s->L + (int64_t)s->gy * TILE * ld;
+        PIGP_TRY(launch_pad(w.L, ld, s->n, s->n, s->npad, s->npad, 1, 1, st, nb, w.sL));
+    double* ytile = w.L + (int64_t)s->gy * TILE * ld;
     {
         ProfScope prof(PROF_MISC, st);
-        k_set_ytile<<<148, 256, 0, st>>>(ytile, ld, s->n, s->npad, y_dev);
+        k_set_ytile<<<dim3(148, nb), 256, 0, st>>>(ytile, ld, s->n, s->npad, y_dev, w.sL);
         count_launch();
     }
     PIGP_CUDA(cudaGetLastError());
@@ -982,10 +1136,10 @@ static int dsolver_enqueue(pigp_dsolver* s, const double* theta_dev, const doubl
     }
     // every rank holds all of L now (the panel flags of every peer were awaited inside rec for all but the final leaf,
     // whose diagonal tile arrives with its DIAG flag)
-    PIGP_TRY(launch_logdet_quad(s->L, ld, s->n, ytile, s->out2, st));
-    k_diag_info<<<1, 1024, 0, st>>>(s->L, ld, s->n, info);
+    PIGP_TRY(launch_logdet_quad(w.L, ld, s->n, ytile, w.out2, st, nb, w.sL, w.sL));
+    k_diag_info<<<dim3(1, nb), 1024, 0, st>>>(w.L, ld, s->n, info, w.sL);
     count_launch();
-    k_finish_nll_d<<<1, 1, 0, st>>>(s->out2, s->n, info, s->err, nll_dev);
+    k_finish_nll_d<<<dim3(1, nb), 1, 0, st>>>(w.out2, s->n, info, s->err, nll_dev);
     count_launch();
     PIGP_CUDA(cudaGetLastError());
     if (c.grad) {
@@ -1007,8 +1161,8 @@ static int dsolver_enqueue(pigp_dsolver* s, const double* theta_dev, const doubl
         // alpha = K^-1 y = Y (L^-1 y), redundantly on every rank
         {
             ProfScope prof(PROF_MISC, st);
-            k_copy_v<<<(unsigned)((s->npad + 255) / 256), 256, 0, st>>>(ytile, s->npad, s->v);
-            k_gemv_upper<<<(unsigned)((s->npad + 7) / 8), 256, 0, st>>>(s->Y, ld, s->npad, s->v, s->alpha);
+            k_copy_v<<<dim3((unsigned)((s->npad + 255) / 256), nb), 256, 0, st>>>(ytile, s->npad, w.v, w.sL);
+            k_gemv_upper<<<dim3((unsigned)((s->npad + 7) / 8), nb), 256, 0, st>>>(c.Y, ld, s->npad, w.v, w.alpha, c.sY);
             count_launch(2);
         }
         PIGP_CUDA(cudaGetLastError());
@@ -1020,30 +1174,32 @@ static int dsolver_enqueue(pigp_dsolver* s, const double* theta_dev, const doubl
             GemmDesc g{};
             g.M = cnt * TILE; g.N = (int)s->npad; g.K = (int)s->npad;
             g.alpha = 1.0; g.beta = 0.0;
-            g.A = s->Y + (int64_t)first * TILE * ld; g.lda = ld; g.a_kcontig = 1;
-            g.B = s->Y; g.ldb = ld; g.b_kcontig = 1;
-            g.C = s->L + (int64_t)first * TILE * ld; g.ldc = ld;
+            g.A = c.Y + (int64_t)first * TILE * ld; g.lda = ld; g.a_kcontig = 1;
+            g.B = c.Y; g.ldb = ld; g.b_kcontig = 1;
+            g.C = w.L + (int64_t)first * TILE * ld; g.ldc = ld;
             g.lower_only = 1; g.kmode = 1;
             g.gen = 1; g.m_ts = s->world; g.m_gt0 = first; g.n_gt0 = 0; g.k_gt0 = 0;
+            set_slots(g, c, c.sY, c.sY, w.sL);
             PIGP_TRY(launch_gemm(g, st));
         }
-        PIGP_TRY(launch_grad(p, s->d_tiles, s->n_tiles, theta_dev, c.early_kinv ? s->Kinv : s->L, ld, s->alpha, s->partials, s->gpart, st));
+        PIGP_TRY(launch_grad(p, s->d_tiles, s->n_tiles, theta_dev, c.early_kinv ? c.Kinv : w.L, ld, w.alpha, w.partials, w.gpart, st,
+                             nb, P, c.early_kinv ? c.sY : w.sL, s->npad, std::max<int64_t>(s->n_tiles, 1) * MAX_THETA, MAX_THETA));
         {
             PeerBufs pb{};
             pb.n = c.npeers;
             for (int q = 0; q < c.npeers; ++q) pb.p[q] = s->peer(c.others[q], s->gslots);
             ProfScope prof(PROF_GRAD, st);
-            k_push_vec<<<1, 32, 0, st>>>(s->gpart, p->theta_len, s->rank, s->gslots, pb);
+            k_push_vec<<<dim3(1, nb), 32, 0, st>>>(w.gpart, p->theta_len, s->rank, w.gslots, pb, (int64_t)s->world * MAX_THETA);
             count_launch();
         }
         PIGP_CUDA(cudaGetLastError());
         PIGP_TRY(signal(c, s->f_grad(s->rank)));
         PIGP_TRY(wait_all(c, s->f_grad(0), st));
-        k_sum_slots<<<1, 32, 0, st>>>(s->gslots, s->world, p->theta_len, grad_dev, info, s->err);
+        k_sum_slots<<<dim3(1, nb), 32, 0, st>>>(w.gslots, s->world, p->theta_len, grad_dev, info, s->err, (int64_t)s->world * MAX_THETA);
         count_launch();
         PIGP_CUDA(cudaGetLastError());
     }
-    if (info_dev) PIGP_CUDA(cudaMemcpyAsync(info_dev, info, sizeof(int32_t), cudaMemcpyDeviceToDevice, st));
+    if (info_dev) PIGP_CUDA(cudaMemcpyAsync(info_dev, info, sizeof(int32_t) * nb, cudaMemcpyDeviceToDevice, st));
     return PIGP_OK;
 }
 

@@ -126,6 +126,10 @@ struct AsmArgs {
     const double* X;    // K^-1, lower triangle
     const double* alpha;
     double* partials;   // [n_tiles][MAX_THETA]
+    // batch: nb slots share the points and the tile list; slot b = blockIdx.y reads and writes its pointers offset by b times
+    // these strides (0: shared by every slot)
+    int nb;
+    int64_t s_theta, s_K, s_X, s_alpha, s_partials;
 };
 
 AsmArgs make_args(const pigp_plan* p, const AsmTile* tiles, const double* theta, double eps, int add_diag);
@@ -141,17 +145,31 @@ __device__ __forceinline__ double diag_addon(const AsmArgs& a, int64_t R, double
     return a.eps;
 }
 
+// the slot's pointers (once, at kernel entry).  The evaluators are instantiated twice, with and without this: the single-slot
+// kernels stay exactly as register-tight as they were (several run at their register cap)
+__device__ __forceinline__ void slot_args(AsmArgs& a) {
+    const int64_t b = blockIdx.y;
+    a.theta += b * a.s_theta;
+    a.K += b * a.s_K;
+    a.X += b * a.s_X;
+    a.alpha += b * a.s_alpha;
+    a.partials += b * a.s_partials;
+}
+
 #endif
 
-// ---- assembly / gradient (pigp_assemble.cu)
+// ---- assembly / gradient (pigp_assemble.cu).  The trailing nb and strides batch a launch over nb slots (one more grid
+// dimension): slot b reads theta_dev + b * s_theta and writes K + b * s_K, and so on.
 int launch_assemble(const pigp_plan* p, const AsmTile* tiles, int64_t n_tiles, const double* theta_dev, double eps,
-                    int add_diag, double* K, int64_t ld, cudaStream_t st);
+                    int add_diag, double* K, int64_t ld, cudaStream_t st, int nb = 1, int64_t s_theta = 0, int64_t s_K = 0);
 // zero-fill + unit diagonal for rows/cols outside the plan's extent, up to rows_pad x cols_pad
 int launch_pad(double* K, int64_t ld, int64_t rows, int64_t cols, int64_t rows_pad, int64_t cols_pad, int unit_diag,
-               int lower_only, cudaStream_t st);
+               int lower_only, cudaStream_t st, int nb = 1, int64_t s_K = 0);
 // partials[n_tiles_lower][MAX_THETA] <- per-tile sums of (X - alpha alpha^T) * dK/dtheta ; then reduce into grad
+// (slot b: grad_out + b * s_grad)
 int launch_grad(const pigp_plan* p, const AsmTile* tiles, int64_t n_tiles, const double* theta_dev, const double* X, int64_t ld,
-                const double* alpha, double* partials, double* grad_out, cudaStream_t st);
+                const double* alpha, double* partials, double* grad_out, cudaStream_t st, int nb = 1, int64_t s_theta = 0,
+                int64_t s_X = 0, int64_t s_alpha = 0, int64_t s_partials = 0, int64_t s_grad = 0);
 // lower-triangle tiles of a symmetric plan whose 128-row tile belongs to `rank` (tile t -> rank t mod world); tiles never
 // straddle a 128-row boundary
 void build_lower_tiles_owned(const pigp_plan* p, int rank, int world, std::vector<AsmTile>& out);
@@ -167,11 +185,18 @@ struct FactorView {
     int32_t* info;   // first failing pivot (may be null)
     int rank, world; // 128-row tile t belongs to rank t mod world
     double* v;       // L^-1 y (npad entries; zeros beyond n): solver only
+    // batch (world = 1): nb matrices factored by the same launches; slot b's L (and v) at + b * sL, its invd at + b * sI,
+    // its info at + b
+    int nb;
+    int64_t sL, sI;
     // first own tile >= a
     int first_own(int a) const { return a + ((rank - a) % world + world) % world; }
     int count_own(int a, int b) const { const int f = first_own(a); return f < b ? (b - f + world - 1) / world : 0; }
 };
 FactorView factor_view(pigp_dsolver* s);
+// pigp_nll_grad_batch on the solver's world = 1 block-cyclic solver (pigp_dist.cu): nb slots, one pass of the schedule
+int dsolver_nll_grad_batch(pigp_dsolver* s, int nb, const double* thetas_dev, const double* y_dev, double eps, double* nll_dev,
+                           double* grad_dev, int32_t* info_dev, void* stream);
 
 // ---- dense linear algebra (pigp_dense.cu)
 struct GemmDesc {
@@ -210,19 +235,27 @@ struct GemmDesc {
     int sig_total, sig_n;
     unsigned long long sig_val;
     unsigned long long* sig_flag[7];
+    // ---- batch: nb (0 is read as 1) independent products of this shape in one launch (grid dimension y = slot); slot b
+    //      works on A + b * sa, B + b * sb, C + b * sc and Lkk + b * sl.  Every choice of kernel variant is made from the
+    //      shape of one slot, so a slot's result does not depend on nb.
+    int nb;
+    int64_t sa, sb, sc, sl;
 };
 int launch_gemm(const GemmDesc& g, cudaStream_t st);
 // factor one 128 x 128 diagonal tile in place; invd receives the four diagonal 32 x 32 blocks of inv(L) only
-int launch_potf2(double* A, int64_t ld, double* invd, int32_t* info, int base, cudaStream_t st);
+// (nb slots: A + b * sA, invd + b * sI, info + b)
+int launch_potf2(double* A, int64_t ld, double* invd, int32_t* info, int base, cudaStream_t st, int nb = 1, int64_t sA = 0,
+                 int64_t sI = 0);
 // complete the inverse tiles c = first + i * stride (i < count) from L_cc and their diagonal blocks; Y != nullptr: also
-// write inv(L_cc)^T into the diagonal tile c of Y (row stride ldy)
+// write inv(L_cc)^T into the diagonal tile c of Y (row stride ldy).  nb slots: L + b * sL, invd + b * sI, Y + b * sY
 int launch_tile_inv(const double* L, int64_t ld, double* invd, int first, int stride, int count, double* Y, int64_t ldy, cudaStream_t st,
-                    int zero_upper = 0);
+                    int zero_upper = 0, int nb = 1, int64_t sL = 0, int64_t sI = 0, int64_t sY = 0);
 // pigp_potrf_lower (pigp_dist.cu: the solver's factorisation over the caller's buffer)
 int potrf_lower(double* A, int64_t ld, int64_t n, int64_t m_extra, double* invd, int32_t* info, cudaStream_t st);
 int potri_lower(const double* L, int64_t ld, int64_t n, const double* invd, double* W, double* X, cudaStream_t st);
-// out[0] = sum_{i<n} log A[i*ld+i]; out[1] = sum_{j<n} v[j]^2  (v = row `vrow` of A)
-int launch_logdet_quad(const double* A, int64_t ld, int64_t n, const double* v, double* out2, cudaStream_t st);
+// out[0] = sum_{i<n} log A[i*ld+i]; out[1] = sum_{j<n} v[j]^2  (nb slots: A + b * sA, v + b * sv, out2 + 2 b)
+int launch_logdet_quad(const double* A, int64_t ld, int64_t n, const double* v, double* out2, cudaStream_t st, int nb = 1,
+                       int64_t sA = 0, int64_t sv = 0);
 // y[i] = sum_j A[i*ld+j] x[j], A (m x n) row-major
 int launch_gemv(const double* A, int64_t ld, int64_t m, int64_t n, const double* x, double* y, cudaStream_t st);
 

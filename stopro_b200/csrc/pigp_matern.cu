@@ -128,9 +128,10 @@ __device__ __forceinline__ double mat_eval(const MatShared& sh, int kind, const 
     return val;
 }
 
-template <int DIM, bool PRODUCT, bool GRAD>
+template <int DIM, bool PRODUCT, bool GRAD, bool BATCH>
 __global__ void __launch_bounds__(256) k_blocks_matern(AsmArgs a, int kind) {
     __shared__ MatShared sh;
+    if (BATCH) slot_args(a);
     const AsmTile tl = a.tiles[blockIdx.x];
     const int tid = threadIdx.x;
     const bool live = tl.desc >= 0;
@@ -238,17 +239,23 @@ __global__ void __launch_bounds__(256) k_blocks_matern(AsmArgs a, int kind) {
     }
 }
 
+template <int DIM, bool PRODUCT, bool GRAD>
+static void launch_k(const AsmArgs& a, int64_t n_tiles, int kind, cudaStream_t st) {
+    const dim3 grid((unsigned)n_tiles, (unsigned)a.nb), block(256);
+    if (a.nb > 1) k_blocks_matern<DIM, PRODUCT, GRAD, true><<<grid, block, 0, st>>>(a, kind);
+    else k_blocks_matern<DIM, PRODUCT, GRAD, false><<<grid, block, 0, st>>>(a, kind);
+}
+
 template <bool GRAD>
 static int launch_t(const pigp_plan* p, const AsmArgs& a, int64_t n_tiles, int kind, cudaStream_t st) {
-    const dim3 grid((unsigned)n_tiles), block(256);
     ProfScope prof(GRAD ? PROF_GRAD : PROF_ASSEMBLE, st);
-    if (p->dim == 1) k_blocks_matern<1, true, GRAD><<<grid, block, 0, st>>>(a, kind);
+    if (p->dim == 1) launch_k<1, true, GRAD>(a, n_tiles, kind, st);
     else if (p->dim == 2) {
-        if (p->product_form) k_blocks_matern<2, true, GRAD><<<grid, block, 0, st>>>(a, kind);
-        else k_blocks_matern<2, false, GRAD><<<grid, block, 0, st>>>(a, kind);
+        if (p->product_form) launch_k<2, true, GRAD>(a, n_tiles, kind, st);
+        else launch_k<2, false, GRAD>(a, n_tiles, kind, st);
     } else {
-        if (p->product_form) k_blocks_matern<3, true, GRAD><<<grid, block, 0, st>>>(a, kind);
-        else k_blocks_matern<3, false, GRAD><<<grid, block, 0, st>>>(a, kind);
+        if (p->product_form) launch_k<3, true, GRAD>(a, n_tiles, kind, st);
+        else launch_k<3, false, GRAD>(a, n_tiles, kind, st);
     }
     count_launch();
     PIGP_CUDA(cudaGetLastError());
@@ -263,11 +270,11 @@ int launch_blocks_matern(const pigp_plan* p, const AsmArgs& a, int64_t n_tiles, 
 
 int preload_matern() {
     PIGP_TRY(upload_tables());
-    PIGP_PRELOAD((k_blocks_matern<1, true, false>)); PIGP_PRELOAD((k_blocks_matern<1, true, true>));
-    PIGP_PRELOAD((k_blocks_matern<2, true, false>)); PIGP_PRELOAD((k_blocks_matern<2, true, true>));
-    PIGP_PRELOAD((k_blocks_matern<2, false, false>)); PIGP_PRELOAD((k_blocks_matern<2, false, true>));
-    PIGP_PRELOAD((k_blocks_matern<3, true, false>)); PIGP_PRELOAD((k_blocks_matern<3, true, true>));
-    PIGP_PRELOAD((k_blocks_matern<3, false, false>)); PIGP_PRELOAD((k_blocks_matern<3, false, true>));
+    PIGP_PRELOAD((k_blocks_matern<1, true, false, false>)); PIGP_PRELOAD((k_blocks_matern<1, true, true, false>));
+    PIGP_PRELOAD((k_blocks_matern<2, true, false, false>)); PIGP_PRELOAD((k_blocks_matern<2, true, true, false>));
+    PIGP_PRELOAD((k_blocks_matern<2, false, false, false>)); PIGP_PRELOAD((k_blocks_matern<2, false, true, false>));
+    PIGP_PRELOAD((k_blocks_matern<3, true, false, false>)); PIGP_PRELOAD((k_blocks_matern<3, true, true, false>));
+    PIGP_PRELOAD((k_blocks_matern<3, false, false, false>)); PIGP_PRELOAD((k_blocks_matern<3, false, true, false>));
     return PIGP_OK;
 }
 

@@ -219,6 +219,27 @@ class Solver:
                                                  int(want_grad), C.addressof(nll), grad.ctypes.data, C.addressof(info)))
         return nll.value, (grad if want_grad else None), info.value
 
+    def nll_grad_batch_host(self, thetas, y, eps, want_grad=True):
+        """NLL (+ gradient) of B hyper-parameter vectors (rows of ``thetas``) in one pass of the factorisation schedule
+        (pigp_nll_grad_batch_host) -> (nll (B,), grad (B, P) or None, info (B,)).  Slot b equals nll_grad_host(thetas[b])
+        bit for bit."""
+        p = self.plan
+        th = np.ascontiguousarray(np.stack([p._theta(t) for t in thetas]))
+        yy = np.ascontiguousarray(np.asarray(y, dtype=np.float64).ravel())
+        if yy.size != p.rows:
+            raise ValueError(f"delta_y has {yy.size} entries, the training set has {p.rows}")
+        nb = len(th)
+        nll = np.empty(nb, dtype=np.float64)
+        grad = np.empty((nb, p.theta_len), dtype=np.float64)
+        info = np.zeros(nb, dtype=np.int32)
+        _lib.check(_lib.lib().pigp_nll_grad_batch_host(self.handle, nb, th.ctypes.data, yy.ctypes.data, float(eps),
+                                                       int(want_grad), nll.ctypes.data, grad.ctypes.data, info.ctypes.data))
+        return nll, (grad if want_grad else None), info
+
+    def nll_grad_batch(self, n_theta, thetas_ptr, y_ptr, eps, nll_ptr, grad_ptr=None, info_ptr=None, stream=None):
+        _lib.check(_lib.lib().pigp_nll_grad_batch(self.handle, int(n_theta), thetas_ptr, y_ptr, float(eps), nll_ptr, grad_ptr,
+                                                  info_ptr, stream))
+
     def nll_grad(self, theta_ptr, y_ptr, eps, nll_ptr, grad_ptr, info_ptr=None, stream=None):
         _lib.check(_lib.lib().pigp_nll_grad(self.handle, theta_ptr, y_ptr, float(eps), nll_ptr, grad_ptr, info_ptr, stream))
 
@@ -229,25 +250,33 @@ class Solver:
                   check_every=16):
         """Device-resident optimize_by_adam loop (pigp_adam_host) -> (theta_hist (n+1, P), loss_hist (n+1,),
         gradnorm_hist (n,), status)."""
+        return self.adam_batch_host([theta0], y, eps, max_iter, lr, stop_eps, ntraining, ridge_alpha=ridge_alpha,
+                                    ridge_in_grad=ridge_in_grad, fixed=fixed, check_every=check_every)[0]
+
+    def adam_batch_host(self, theta0s, y, eps, max_iter, lr, stop_eps, ntraining, ridge_alpha=0.0, ridge_in_grad=True,
+                        fixed=None, check_every=16):
+        """adam_host from every row of ``theta0s`` at once (pigp_adam_batch_host: one batched evaluation per iteration)
+        -> list over starts of (theta_hist, loss_hist, gradnorm_hist, status), each equal to adam_host from that start."""
         p = self.plan
-        th = p._theta(theta0)
+        th = np.ascontiguousarray(np.stack([p._theta(t) for t in theta0s]))
         yy = np.ascontiguousarray(np.asarray(y, dtype=np.float64).ravel())
-        P = p.theta_len
-        theta_hist = np.empty((max_iter + 1, P), dtype=np.float64)
-        loss_hist = np.empty(max_iter + 1, dtype=np.float64)
-        norm_hist = np.empty(max_iter, dtype=np.float64)
+        nb, P = len(th), p.theta_len
+        theta_hist = np.empty((nb, max_iter + 1, P), dtype=np.float64)
+        loss_hist = np.empty((nb, max_iter + 1), dtype=np.float64)
+        norm_hist = np.empty((nb, max_iter), dtype=np.float64)
         mask = None
         if fixed is not None and len(fixed):
             mask = np.zeros(P, dtype=np.int32)
             mask[np.asarray(fixed, dtype=int)] = 1
-        n_done, status = C.c_int32(), C.c_int32()
-        _lib.check(_lib.lib().pigp_adam_host(self.handle, th.ctypes.data, yy.ctypes.data, float(eps), int(max_iter), float(lr),
-                                             float(stop_eps), float(ntraining), float(ridge_alpha), int(ridge_in_grad),
-                                             mask.ctypes.data if mask is not None else None, int(check_every),
-                                             theta_hist.ctypes.data, loss_hist.ctypes.data, norm_hist.ctypes.data,
-                                             C.addressof(n_done), C.addressof(status)))
-        n = n_done.value
-        return theta_hist[:n + 1].copy(), loss_hist[:n + 1].copy(), norm_hist[:n].copy(), status.value
+        n_done = np.zeros(nb, dtype=np.int32)
+        status = np.zeros(nb, dtype=np.int32)
+        _lib.check(_lib.lib().pigp_adam_batch_host(self.handle, nb, th.ctypes.data, yy.ctypes.data, float(eps), int(max_iter),
+                                                   float(lr), float(stop_eps), float(ntraining), float(ridge_alpha),
+                                                   int(ridge_in_grad), mask.ctypes.data if mask is not None else None,
+                                                   int(check_every), theta_hist.ctypes.data, loss_hist.ctypes.data,
+                                                   norm_hist.ctypes.data, n_done.ctypes.data, status.ctypes.data))
+        return [(theta_hist[b, :n + 1].copy(), loss_hist[b, :n + 1].copy(), norm_hist[b, :n].copy(), int(status[b]))
+                for b, n in enumerate(n_done)]
 
     def predict_host(self, mixed, test, theta, y, eps, full_cov=True):
         mu, cov, info = self.predict_batch_host(mixed, test, [theta], y, eps, full_cov=full_cov)

@@ -7,6 +7,8 @@ eps = 1e-8), history lists of theta / loss / gradient norm, the two-in-a-row pla
 ONE factorisation (``f.value_and_grad`` of stopro_b200's logposterior) instead of func + dfunc assembling and
 factorising K twice per step (:148-150); and when the loss is stopro_b200's logposterior over a GP model the whole loop
 runs on the device (``_device_loop`` -> pigp_adam_host), the host loop below being the fallback.  The optional scipy pre-stage is delegated to scipy.optimize.minimize.
+``optimize_by_adam_many`` runs optimize_by_adam from several starting points (multi-start fitting: the marginal
+likelihood is not convex in theta); on the device all starts share one batched evaluation per iteration.
 """
 import numpy as np
 
@@ -19,21 +21,30 @@ def _value_and_grad(f, df):
     return lambda p, *args: (f(p, *args), df(p, *args))
 
 
-def _device_loop(f, df, init, params_optimization, ntraining, index_fixed, args):
-    """The whole Adam loop on the device (pigp_adam_host) when the loss is stopro_b200's logposterior over a GP model:
-    theta, the moments and the histories stay in HBM, evaluation and update are enqueued back to back and the host only
-    looks at the stop flag every few iterations.  Same lists and exceptions as the host loop below.  Not used with a
-    scipy pre-stage, with print_process (per-step run.out lines) or with params_optimization["device_loop"] = False."""
+def _device_kwargs(f, df, params_optimization, ntraining, index_fixed, method):
+    """Arguments of GPmodel.adam_device / adam_device_many, or None when the device loop does not apply: the loss is not
+    stopro_b200's logposterior over a GP model, or there is a scipy pre-stage, print_process (per-step run.out lines) or
+    params_optimization["device_loop"] = False."""
     model = getattr(f, "model", None)
-    if (model is None or not hasattr(model, "adam_device") or not params_optimization.get("device_loop", True)
+    if (model is None or not hasattr(model, method) or not params_optimization.get("device_loop", True)
             or params_optimization.get("print_process", False) or not params_optimization.get("maxiter_GD")
             or (params_optimization.get("maxiter_scipy") or [0])[0]):
         return None
     # jit(grad(func)) differentiates the ridge term; the explicit-derivative scripts (df = gp.d_logposterior) drop it
     explicit = getattr(df, "__func__", None) is getattr(type(model), "d_logposterior", None) and df is not None
-    out = model.adam_device(init, *args, max_iter=params_optimization["maxiter_GD"], lr=params_optimization["lr"],
-                            stop_eps=params_optimization["eps"], ntraining=ntraining,
-                            ridge_alpha=getattr(f, "ridge_alpha", 0.0), ridge_in_grad=not explicit, fixed=index_fixed or None)
+    return dict(max_iter=params_optimization["maxiter_GD"], lr=params_optimization["lr"], stop_eps=params_optimization["eps"],
+                ntraining=ntraining, ridge_alpha=getattr(f, "ridge_alpha", 0.0), ridge_in_grad=not explicit,
+                fixed=index_fixed or None)
+
+
+def _device_loop(f, df, init, params_optimization, ntraining, index_fixed, args):
+    """The whole Adam loop on the device (pigp_adam_host) when the loss is stopro_b200's logposterior over a GP model:
+    theta, the moments and the histories stay in HBM, evaluation and update are enqueued back to back and the host only
+    looks at the stop flag every few iterations.  Same lists and exceptions as the host loop below."""
+    kw = _device_kwargs(f, df, params_optimization, ntraining, index_fixed, "adam_device")
+    if kw is None:
+        return None
+    out = f.model.adam_device(init, *args, **kw)
     if out is None:
         return None
     theta_hist, loss_hist, norms, status = out
@@ -127,3 +138,47 @@ def optimize_by_adam(f, df, hf, init, params_optimization, *args):
         else:
             converged_once = False
     return theta[-1], loss, theta, norms
+
+
+# device status of pigp_adam_host -> status of optimize_by_adam_many; the exception messages of optimize_by_adam
+_STATUS = {0: "max_iter", 1: "converged", 2: "grad_nan", 3: "theta_nan", 4: "initial_nan"}
+_RAISED = {"loss is nan at the initial hyper-parameters": "initial_nan", "gradient of loss became nan": "grad_nan",
+           "theta became nan": "theta_nan"}
+
+
+def optimize_by_adam_many(f, df, hf, inits, params_optimization, *args):
+    """optimize_by_adam from every starting point in ``inits`` -> one (theta_final, loss, theta_hist, norms, status) per
+    start, status one of "max_iter", "converged", "grad_nan", "theta_nan" and "initial_nan".  A start that
+    optimize_by_adam would raise for reports that status with None in place of its results; no start raises.  On the
+    device (GPmodel.adam_device_many) every start gets exactly the results optimize_by_adam gives it alone, from one
+    batched evaluation per iteration; elsewhere optimize_by_adam runs once per start."""
+    r_train = args[0]
+    ntraining = sum(np.shape(r)[0] for r in r_train)
+    inits = [np.asarray(x, dtype=np.float64).copy() for x in inits]
+    index_fixed = params_optimization.get("index_fixed")
+    kw = _device_kwargs(f, df, params_optimization, ntraining, index_fixed, "adam_device_many")
+    outs = f.model.adam_device_many(inits, *args, **kw) if kw is not None else None
+    if outs is not None:
+        res = []
+        for theta_hist, loss_hist, norms, status in outs:
+            st = _STATUS[status]
+            if st in _RAISED.values():
+                res.append((None, None, None, None, st))
+                continue
+            theta = [t.copy() for t in theta_hist]
+            res.append((theta[-1], [float(v) for v in loss_hist], theta, [float(v) for v in norms], st))
+        return res
+    res = []
+    eps = params_optimization["eps"]
+    for x in inits:
+        try:
+            theta_final, loss, theta, norms = optimize_by_adam(f, df, hf, x, params_optimization, *args)
+        except Exception as e:
+            if str(e) not in _RAISED:
+                raise
+            res.append((None, None, None, None, _RAISED[str(e)]))
+            continue
+        # the loop stops early only on the two-in-a-row plateau rule, checked from the third step on
+        conv = len(norms) >= 3 and abs(loss[-1] - loss[-2]) < eps and abs(loss[-2] - loss[-3]) < eps
+        res.append((theta_final, loss, theta, norms, "converged" if conv else "max_iter"))
+    return res
